@@ -2,6 +2,7 @@
 """bench.py -- benchmarks of the Reachy2 symbolic IK hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload all|symik|symik_f32|discrete|continuous|reachmap]
+                    [--dump-outputs DIR]
 
 The headline workload `symik` = BASELINE.json configs[1], the configuration the metric is quoted on: 1 M FK-sampled poses per
 arm (r_arm and l_arm), FP64, reachability flag + theta interval + 7 joints at theta_interval[0] + elbow position.  One *step* =
@@ -21,6 +22,13 @@ ms_per_step, roofline, parity and e2e, under torchrun too, so that the scaling r
   rank 0 only.
 * N > 1: launched by torchrun, one rank per GPU, contiguous slices of the batch per rank, no data-path collective (weak
   scaling); the reach map shards orientations and all-reduces the count volume (strong scaling).
+* `--dump-outputs DIR`: after the timed steps, rank 0 writes what the headline workload's last timed step gave it (under
+  torchrun its slice of the batch; the all-reduced volume for the reach map) to
+  DIR/<name>.npy, finite values only (NaN / inf entries as 0, marked in DIR/<name>_nonfinite.npy), a fixed sample of rows
+  when the outputs exceed 48 MiB.  The inputs are seeded, so two builds run with the same arguments can be compared output
+  for output.
+
+The benchmark writes nothing into the source tree (it may be read-only): no bytecode cache, no build.
 """
 from __future__ import annotations
 
@@ -35,6 +43,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True   # the package, the oracle and the scripts it imports live in the (possibly read-only) tree
 REPO = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, REPO)
 
@@ -212,6 +221,10 @@ class Symik:
             o = self.outs[arm]
             self.solvers[arm].solve_into(self.dpose[arm], self.kind, None, None, o["reach"], o["state"], o["interval"], o["joints"], o["elbow"])
         return 2
+
+    def outputs(self):
+        names = {"reach": "reachable", "state": "state", "interval": "theta_interval", "joints": "joints", "elbow": "elbow"}
+        return {f"{arm}_{names[k]}": t for arm in ARMS for k, t in self.outs[arm].items()}
 
     def e2e_setup(self, torch):
         n = self.POSES_PER_ARM
@@ -457,6 +470,9 @@ class Discrete:
         self.out = self.ctl.symbolic_inverse_kinematics_batch("r_arm", self.dM, "discrete", out=self.out)
         return 1
 
+    def outputs(self):
+        return dict(zip(("joints", "reachable", "state", "emergency_bits"), self.out))
+
     def e2e_setup(self, torch):
         self.host_in = torch.from_numpy(self.poses).reshape(self.N, 16).pin_memory()
         self.e2e_out = self.ctl.alloc_host_outputs("discrete", self.N)
@@ -545,6 +561,14 @@ class Continuous:
         self.st.copy_(self.st0)
         self.out = self.ctl.symbolic_inverse_kinematics_batch("r_arm", self.dM, "continuous", states=self.st, out=self.out)
         return 1
+
+    def outputs(self):
+        import torch
+
+        st = self.out[3]                                      # (T, 80) bytes of _abi.TRAJ_STATE_DTYPE per trajectory
+        f64, i32 = st[:, :64].view(torch.float64), st[:, 64:].view(torch.int32)
+        return {"joints": self.out[0], "reachable": self.out[1], "state": self.out[2], "final_previous_theta": f64[:, 0],
+                "final_previous_sol": f64[:, 1:], "final_emergency_stop": i32[:, 2], "final_emergency_bits": i32[:, 3]}
 
     def e2e_setup(self, torch):
         # a bounded slice of the trajectories goes host -> device -> host each e2e step
@@ -662,6 +686,9 @@ class ReachMap:
         e[1].record()
         self._events.append({"t0": e[0], "t1": e[1], "k": [(e[0], e[1])]})
         return 1
+
+    def outputs(self):
+        return {"counts": self.out}
 
     def phase_times(self, env, steps):
         """Kernel time (sum of the slab kernels) and what the all-reduce adds to the step beyond it, by events on the
@@ -875,9 +902,44 @@ class Env:
         return float(t.item())
 
 
-def run_workload(env: Env, wl, steps: int, warmup: int, headline: bool, cpu_baseline: bool):
+DUMP_BYTES = 48 << 20     # --dump-outputs writes at most this much (float32 / float64 .npy payloads)
+DUMP_SEED = 0
+
+
+def dump_outputs(wl, dirname: str) -> dict:
+    """Write what the last timed step computed as <dirname>/<name>.npy: float arrays in their own precision, flags, states
+    and counts as float32 (exact).  Every file holds finite values only: the solver returns NaN joints / interval / elbow
+    for a pose it cannot reach, so each float output is written with those entries set to 0 beside
+    <name>_nonfinite.npy (float32, 1 where the caller receives NaN or inf), which together say exactly what was returned.
+    When the outputs exceed DUMP_BYTES, every array keeps the same fixed, seeded sample of rows along its first axis
+    (poses, trajectories or voxel planes), sorted; arrays of equal length share the sample."""
+    import torch
+
+    outs = wl.outputs()
+    total = sum(t.numel() * ({torch.float64: 8 + 4, torch.float32: 4 + 4}.get(t.dtype, 4)) for t in outs.values())
+    frac = min(1.0, DUMP_BYTES / total)
+    os.makedirs(dirname, exist_ok=True)
+    rows = {}
+    for name, t in outs.items():
+        n = t.shape[0]
+        k = int(n * frac)
+        if k < n:
+            idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, k, replace=False))
+            t = t.index_select(0, torch.from_numpy(idx).to(t.device))
+        a = t.cpu().numpy()
+        if a.dtype in (np.float32, np.float64):
+            bad = ~np.isfinite(a)
+            np.save(os.path.join(dirname, name + "_nonfinite.npy"), bad.astype(np.float32))
+            a = np.where(bad, a.dtype.type(0), a)
+        np.save(os.path.join(dirname, name + ".npy"), a if a.dtype in (np.float32, np.float64) else a.astype(np.float32))
+        rows[name] = [k, n]
+    return {"dir": os.path.abspath(dirname), "rows_written_of_total": rows, "sample_seed": DUMP_SEED if frac < 1.0 else None}
+
+
+def run_workload(env: Env, wl, steps: int, warmup: int, cpu_baseline: bool, dump_dir: str | None = None):
     """Time one workload: W warm-up steps, exactly K timed steps (barrier + synchronize on both sides, CUDA events on the
-    launching stream, max over ranks), the end-to-end leg, the parity spot check, the rooflines.  Returns the record."""
+    launching stream, max over ranks), the end-to-end leg, the parity spot check, the rooflines.  Returns the record.
+    dump_dir: rank 0 writes the outputs of the last timed step there (dump_outputs)."""
     import contextlib
 
     torch, dev, rank, world = env.torch, env.dev, env.rank, env.world
@@ -904,23 +966,11 @@ def run_workload(env: Env, wl, steps: int, warmup: int, headline: bool, cpu_base
            "scaling": getattr(wl, "scaling", "weak"),
            "dtype": getattr(wl, "dtype", "f32" if getattr(wl, "fp32", False) else "f64"), "config": wl.config(world),
            "gpu_launches": launches * getattr(wl, "KERNELS_PER_PASS", 1), "clocks": clocks.summary()}
+    if dump_dir is not None and rank == 0:     # before phase_times: under torchrun it runs the reach map again
+        rec["dump_outputs"] = dict(dump_outputs(wl, dump_dir), rank=rank, world_size=world,
+                                   covers="this rank's share of the step" if world > 1 else "the whole step")
     if hasattr(wl, "phase_times"):
         rec.update(wl.phase_times(env, steps))
-
-    # a sustained run of the headline kernel beside the K-step burst (the driver's K = 20 steps are 3 ms: no clock sample
-    # can fall inside, and the power limit is never reached)
-    if headline:
-        n_sus = max(steps, 1500)
-        with ClockSampler(env.local_rank) as cs:
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record()
-            for _ in range(n_sus):
-                wl.step()
-            e1.record()
-            env.barrier()
-        ms_sus = env.max_over_ranks(e0.elapsed_time(e1))
-        rec["sustained"] = {"steps": n_sus, "value": units_per_step * n_sus / (ms_sus * 1e-3), "ms_per_step": ms_sus / n_sus,
-                            "clocks": cs.summary()}
 
     # ---- end to end through the public facade with pinned host buffers (copies inside the timed region)
     e2e_info = wl.e2e_setup(torch)
@@ -1063,9 +1113,14 @@ def main() -> int:
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="all", choices=["all"] + sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the headline workload's last timed step to DIR/<name>.npy, NaN / inf as 0 and "
+                         "marked in DIR/<name>_nonfinite.npy (about 48 MiB at most)")
     args = ap.parse_args()
     names = ["symik", "symik_f32", "discrete", "continuous", "reachmap"] if args.workload == "all" else [args.workload]
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the GPU path's outputs; the reference arm keeps none")
         return run_reference(args, names)
     head = WORKLOADS[names[0]]()
     default_steps = {"symik": 2000, "symik_f32": 2000, "discrete": 50, "continuous": 5, "reachmap": 5}[head.name]
@@ -1091,12 +1146,12 @@ def main() -> int:
 
     binding = hostmem.bind_to_gpu_numa(local_rank)     # pinned buffers and copy threads next to this rank's GPU
     env = Env(torch, dist, torch.device("cuda", local_rank), rank, world, local_rank)
-    rec = run_workload(env, head, args.steps, args.warmup, headline=True, cpu_baseline=not args.no_cpu_baseline)
+    rec = run_workload(env, head, args.steps, args.warmup, cpu_baseline=not args.no_cpu_baseline, dump_dir=args.dump_outputs)
     subs = {}
     for name in names[1:]:
         k, w = SUB_STEPS[name]
         try:
-            subs[name] = run_workload(env, WORKLOADS[name](), k, w, headline=False, cpu_baseline=not args.no_cpu_baseline)
+            subs[name] = run_workload(env, WORKLOADS[name](), k, w, cpu_baseline=not args.no_cpu_baseline)
         except Exception as e:   # a sub-record can only add a key: the headline line stands without it
             import traceback
 

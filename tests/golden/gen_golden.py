@@ -9,6 +9,9 @@ Runs only in the build container, where the reference checkout is mounted read-o
 Oracle of record = reference source + this container's numpy / scipy (versions are stored
 in every file; the reference pins scipy == 1.8.0, this container has scipy 1.18.1).
 
+Every file stays below 1 MB: symik_random_<arm>.npz, symik_ctor.npz and symik_elbow.npz keep a fixed, seeded subset
+of the poses solved here (golden_subset.py says which rows and why the tests still find their blocks).
+
 Reference quirk handled here (SURVEY.md A.6.1): ``get_joints`` mutates the solver when the
 elbow projection fires, so every ``get_joints`` below is preceded by a fresh ``is_reachable``.
 """
@@ -37,6 +40,7 @@ from reachy2_symbolic_ik.symbolic_ik import SymbolicIK  # noqa: E402
 from reachy2_symbolic_ik.utils import get_ik_parameters_from_urdf  # noqa: E402
 
 from reachy2_symbolic_ik_b200 import fk  # noqa: E402
+import golden_subset  # noqa: E402  (this directory: sys.path[0] when run as a script)
 
 STATE_CODES = {
     "reachable": 0,
@@ -168,10 +172,9 @@ def gen_symik_random(n_fk=3000, n_task=3000):
                          interval[:, 1] + 2 * np.pi - interval[:, 0])
         theta2 = np.where(flag, interval[:, 0] + u * width, 0.0)
         _, _, _, joints2, elbow2 = run_symik(ik, gp, theta2)
-        np.savez_compressed(
-            os.path.join(HERE, f"symik_random_{arm}.npz"), **META, M=M, goal_pose=gp, reachable=flag, state=state,
-            interval=interval, joints=joints, elbow=elbow, theta2=theta2, joints_theta2=joints2, elbow_theta2=elbow2,
-            n_fk=n_fk, n_task=n_task)
+        out = dict(META, M=M, goal_pose=gp, reachable=flag, state=state, interval=interval, joints=joints, elbow=elbow,
+                   theta2=theta2, joints_theta2=joints2, elbow_theta2=elbow2, n_fk=n_fk, n_task=n_task)
+        np.savez_compressed(os.path.join(HERE, f"symik_random_{arm}.npz"), **golden_subset.symik_random(out, seed))
         print(arm, "symik_random: reachable", flag.mean(), "states", np.bincount(state, minlength=8))
 
 
@@ -227,7 +230,7 @@ def gen_symik_ctor(n_fk=900, n_task=900):
                         pre + "elbow": elbow, pre + "theta2": theta2, pre + "joints_theta2": joints2,
                         pre + "elbow_theta2": elbow2})
             print(arm, "symik_ctor", name, "reachable", flag.mean(), "states", np.bincount(state, minlength=8))
-    np.savez_compressed(os.path.join(HERE, "symik_ctor.npz"), **out)
+    np.savez_compressed(os.path.join(HERE, "symik_ctor.npz"), **golden_subset.symik_ctor(out))
 
 
 def gen_symik_big_euler(n=800):
@@ -330,7 +333,7 @@ def gen_symik_elbow(n_fk=400, n_task=400, K=4):
                     pre + "nl_joints": nl_joints, pre + "nl_elbow": nl_elbow, pre + "nl_elbow_len": nl_elbow_len})
         print(arm, "symik_elbow: reachable", flag.mean(), "projection fired (limits)", (gj_elbow_len[flag] == 3).mean(),
               "(no limits)", (nl_elbow_len == 3).mean(), "limited by wrist", (state == 4).mean())
-    np.savez_compressed(os.path.join(HERE, "symik_elbow.npz"), **out)
+    np.savez_compressed(os.path.join(HERE, "symik_elbow.npz"), **golden_subset.symik_elbow(out, n_fk, n_task))
 
 
 def gen_ctl_ctor(n_variants=6):

@@ -67,7 +67,8 @@ def test_scalar_call_sequence(oracle, arm):
     ik = SymbolicIK(arm=arm)
     cfg = oracle.arm_config(arm)
     P = g[f"{arm}_goal_pose"]
-    idx = np.r_[0:60, 400:460, len(P) - 24:len(P)]
+    nf = int(g["n_fk"])                                   # FK-sampled poses first, then task space, then the 24 named poses
+    idx = np.r_[0:60, nf:nf + 60, len(P) - 24:len(P)]
     singular = len(P) - 24 + 10                           # the fully stretched arm (see test_named_poses)
     tol = 1e-9
     n_proj = n_plain = 0

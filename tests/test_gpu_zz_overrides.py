@@ -205,9 +205,10 @@ def test_constructor_variants(oracle, arm, variant):
         rep.close("joints@theta2", res2.joints, g[pre + "joints_theta2"])
         rep.close("elbow@theta2", res2.elbow, g[pre + "elbow_theta2"])
         rep.check(max_ill_fraction=0.03)
-    # is_reachable_no_limits (symbolic_ik.py:85-119) on the first / last 250 poses
+    # is_reachable_no_limits (symbolic_ik.py:85-119) on the first / last h poses
     M = g[f"{arm}_M"]
-    sel = np.r_[0:250, len(M) - 250:len(M)]
+    h = len(g[pre + "nl_theta"]) // 2
+    sel = np.r_[0:h, len(M) - h:len(M)]
     Mc, th = np.ascontiguousarray(M[sel]), g[pre + "nl_theta"]
     ill = ill_conditioned_mask(lambda p: oracle.symik_no_limits_batch(ocfg, p.reshape(Mc.shape), th), Mc.reshape(len(sel), -1))
     nj, ne = ik.is_reachable_no_limits_batch(Mc, th)

@@ -103,9 +103,10 @@ def test_constructor_variants(hs, oracle, arm, variant):
         rep.close("joints@theta2", j2, g[pre + "joints_theta2"])
         rep.close("elbow@theta2", e2, g[pre + "elbow_theta2"])
         rep.check(max_ill_fraction=0.03)
-    # is_reachable_no_limits (symbolic_ik.py:85-119) on the first / last 250 poses (FK-sampled / task space)
+    # is_reachable_no_limits (symbolic_ik.py:85-119) on the first / last h poses (FK-sampled / task space)
     Mn = g[f"{arm}_M"]
-    sel = np.r_[0:250, len(Mn) - 250:len(Mn)]
+    h = len(g[pre + "nl_theta"]) // 2
+    sel = np.r_[0:h, len(Mn) - h:len(Mn)]
     Mc = np.ascontiguousarray(Mn[sel])
     th = np.ascontiguousarray(g[pre + "nl_theta"])
     nj = np.empty((len(sel), 7)); ne = np.empty((len(sel), 3))

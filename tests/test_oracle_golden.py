@@ -95,8 +95,9 @@ def test_constructor_variants(oracle, arm, variant):
         rep.close("joints@theta2", j2, g[pre + "joints_theta2"])
         rep.close("elbow@theta2", e2, g[pre + "elbow_theta2"])
         rep.check(max_ill_fraction=0.03)
-        # is_reachable_no_limits (symbolic_ik.py:85-119) on the first / last 250 poses (FK-sampled / task space)
-        sel = np.r_[0:250, len(P) - 250:len(P)]
+        # is_reachable_no_limits (symbolic_ik.py:85-119) on the first / last h poses (FK-sampled / task space)
+        h = len(g[pre + "nl_theta"]) // 2
+        sel = np.r_[0:h, len(P) - h:len(P)]
         nj, ne = oracle.symik_no_limits_batch(cfg, P[sel], g[pre + "nl_theta"])
         ill_nl = ill_conditioned_mask(lambda p: oracle.symik_no_limits_batch(cfg, p.reshape(P[sel].shape), g[pre + "nl_theta"]),
                                       P[sel].reshape(len(sel), -1))
@@ -150,7 +151,8 @@ def test_scalar_call_sequence_record(oracle, arm):
     g = load("symik_elbow.npz")
     cfg = oracle.arm_config(arm)
     P = g[f"{arm}_goal_pose"]
-    idx = np.r_[0:120, 400:520, len(P) - 24:len(P)]       # FK-sampled, task-space and the named poses
+    nf = int(g["n_fk"])
+    idx = np.r_[0:120, nf:nf + 120, len(P) - 24:len(P)]  # FK-sampled, task-space and the named poses
     singular = len(P) - 24 + 10                           # the fully stretched arm: a true singularity (see test_named_poses)
     worst = 0.0
     for i in idx[idx != singular]:
