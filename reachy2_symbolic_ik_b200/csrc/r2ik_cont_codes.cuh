@@ -204,6 +204,36 @@ R2IK_HD void cont_apply_windings(unsigned code, double *row) {
   }
 }
 
+// Raw joints of waypoint k (kind c, not INVALID) at its rate-limited theta: get_joints by the straight-line route + the
+// Orbita3D limit.  Returns true (serial) when get_joints met a degenerate input -- an exact singularity needs previous_sol,
+// so the finish scan redoes the waypoint in order -- or when the test hook force_serial_mod = m > 0 picks the waypoint
+// (ABI parameter test_force_serial_mod: every m-th waypoint takes the serial route although it does not need it, so that
+// the route is exercised on ordinary data).
+R2IK_HD bool cont_raw_joints_item(const ArmConst &A, const R2ikCtlParams &par, const double *row, int c, const double *theta,
+                                  size_t k, int force_serial_mod, double j[7]) {
+  Solve S;
+  double pos[3];
+  load_pose<R2IK_POSE_MAT4>(row, true, pos, S.R);
+  if (c == R2IK_WP_UNREACHABLE) is_reachable_R<true>(A, pos, S);
+  else circle_of_reachable(A, pos, S);   // reachable (phase 1 decided): the elbow circle is all get_joints needs
+  double st, ct, E[3];
+  sincos_any(*theta, st, ct);
+  bool serial = !get_joints_impl<false>(A, S, ct, st, 0.0, 0.0, j, E);
+  if (force_serial_mod > 0 && k % (size_t)force_serial_mod == 0) serial = true;
+  if (!serial) limit_orbita3d_wrist(j, par.orbita3d_max_angle);
+  return serial;
+}
+
+// The serial get_joints of one waypoint (ctl:369-393 with previous_sol[0], [2]): the rare route.
+R2IK_HD void cont_serial_joints(const ArmConst &A, const R2ikCtlParams &par, const double *row, int kind, double theta,
+                                double prev0, double prev2, double j[7]) {
+  Solve S;
+  double pos[3];
+  load_pose<R2IK_POSE_MAT4>(row, true, pos, S.R);
+  if (kind != R2IK_WP_UNREACHABLE) is_reachable_R<false>(A, pos, S);
+  cont_raw_joints(A, par, kind, pos, S, theta, prev0, prev2, j);
+}
+
 // A whole trajectory in one segment (tests/hostsim).
 template <typename SerialFn>
 R2IK_HD void cont_finish_codes_trajectory(int W, const double *current_joints, R2ikTrajState &cs, const double *thetas,
@@ -218,18 +248,11 @@ R2IK_HD void cont_finish_codes_trajectory(int W, const double *current_joints, R
 }  // namespace r2ik
 
 #if defined(__CUDACC__)
-// The serial get_joints of one waypoint (ctl:369-393 with previous_sol[0], [2]): out of line, the rare route.
+// cont_serial_joints, out of line on the device: the rare route
 __device__ __noinline__ void tile_serial_joints(const r2ik::ArmConst &A, const R2ikCtlParams &par, const double *M, int kind, double theta,
                                                 double prev0, double prev2, double *j) {
-  using namespace r2ik;
-  double m[16];
-  load_mat4(M, m);
-  Solve S;
-  double pos[3] = {m[3], m[7], m[11]};
-  rotation_from_mat4(m, true, S.R);
-  if (kind != R2IK_WP_UNREACHABLE) is_reachable_R<false>(A, pos, S);
   double jj[7];
-  cont_raw_joints(A, par, kind, pos, S, theta, prev0, prev2, jj);
+  r2ik::cont_serial_joints(A, par, M, kind, theta, prev0, prev2, jj);
   for (int q = 0; q < 7; ++q) j[q] = jj[q];
 }
 
@@ -270,23 +293,7 @@ k_cont_raw_joints_codes(const __grid_constant__ r2ik::ArmConst A, const __grid_c
       c = sb == R2IK_STATE_INVALID_ROTATION ? R2IK_WP_INVALID
           : (sb == R2IK_STATE_EMPTY || sb == R2IK_STATE_LIMITED_BY_SHOULDER) ? R2IK_WP_TARGET : R2IK_WP_UNREACHABLE;
     }
-    if (c != R2IK_WP_INVALID) {
-      double m[16];
-      load_mat4(M + 16 * k, m);
-      Solve S;
-      double pos[3] = {m[3], m[7], m[11]};
-      rotation_from_mat4(m, true, S.R);
-      if (c == R2IK_WP_UNREACHABLE) is_reachable_R<true>(A, pos, S);
-      else circle_of_reachable(A, pos, S);   // reachable (phase 1 decided): the elbow circle is all get_joints needs
-      double st, ct, E[3];
-      sincos_any(ws[k], st, ct);
-      // straight-line get_joints only; a degenerate input (exact singularity: needs previous_sol) is left to the scan
-      serial = !get_joints_impl<false>(A, S, ct, st, 0.0, 0.0, j, E);
-      // test hook (ABI parameter test_force_serial_mod = m > 0): every m-th waypoint takes the serial route although it
-      // does not need it, so that the route is exercised on ordinary data
-      if (force_serial_mod > 0 && k % (size_t)force_serial_mod == 0) serial = true;
-      if (!serial) limit_orbita3d_wrist(j, par.orbita3d_max_angle);
-    }
+    if (c != R2IK_WP_INVALID) serial = cont_raw_joints_item(A, par, M + 16 * k, c, ws + k, k, force_serial_mod, j);
   }
   const bool ordinary = active && c != R2IK_WP_INVALID && !serial;
 #pragma unroll

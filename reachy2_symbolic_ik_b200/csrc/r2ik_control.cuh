@@ -259,6 +259,18 @@ R2IK_HD double ctor_previous_theta(const ArmConst &A, Solve &S, const double *ro
   return (low + high) / 2;
 }
 
+// ControlIK.__init__'s seed of previous_theta (ctl:142-159): is_reachable_no_limits on the current pose (identity snap of
+// ctl:142), then the constructor's form of the ternary search.  NaN for a pose without an elbow circle.
+R2IK_HD double ctl_ctor_theta(const ArmConst &A, const double *current_pose, const double *rows, int n_rows,
+                              double preferred_theta) {
+  Solve S;
+  const double cpos[3] = {current_pose[3], current_pose[7], current_pose[11]};
+  double theta = NAN;
+  if (rotation_from_mat4(current_pose, true, S.R) && is_reachable_R<true>(A, cpos, S).state == R2IK_STATE_REACHABLE)
+    theta = ctor_previous_theta(A, S, rows, n_rows, preferred_theta);
+  return theta;
+}
+
 // Selection + joints + safety for one pose whose is_reachable result is already known.
 // Shared tail of the discrete path (ctl:454-462).
 R2IK_HD int discrete_finish(const ArmConst &A, const R2ikCtlParams &par, Solve &S, bool found, double theta,
@@ -271,6 +283,53 @@ R2IK_HD int discrete_finish(const ArmConst &A, const R2ikCtlParams &par, Solve &
     for (int i = 0; i < 7; ++i) joints[i] = current_joints[i];
   }
   return safety_checks(joints, prev_joints, par.orbita3d_max_angle);
+}
+
+// Discrete mode, per pose (k_ctl_discrete, k_ctl_discrete_scan and the three passes of r2ik_discrete_compact.cuh).
+// Classify: the rotation with the near-identity snap (ctl:212-217), is_reachable, and for a reachable pose the
+// preferred theta first (utl:357-364); a reachable pose without that shortcut needs the K-sample search.  false:
+// invalid rotation (rc.state = INVALID_ROTATION).
+R2IK_HD bool disc_classify(const ArmConst &A, const R2ikCtlParams &par, const double *row, Solve &S, Reach &rc,
+                           bool &shortcut, bool &need_search) {
+  double pos[3];
+  shortcut = false;
+  need_search = false;
+  rc.state = R2IK_STATE_INVALID_ROTATION;
+  rc.literal = false;
+  if (!load_pose<R2IK_POSE_MAT4>(row, true, pos, S.R)) return false;
+  rc = is_reachable_R<false>(A, pos, S);
+  if (rc.state == R2IK_STATE_REACHABLE) {
+    shortcut = preferred_theta_works(A, S, rc.i0, rc.i1, par.preferred_theta);
+    need_search = !shortcut;
+  }
+  return true;
+}
+
+// The K samples of a pose's search (utl:366-375); the elbow tests P.T are the caller's
+R2IK_HD SearchPlan disc_search_plan(const R2ikCtlParams &par, double i0, double i1) {
+  SearchPlan P;
+  P.preferred_theta = par.preferred_theta;
+  double start, stop;
+  search_range(i0, i1, start, stop);
+  P.L = make_linspace(start, stop, par.nb_search_points);
+  return P;
+}
+// ... with the elbow tests of the solved pose
+R2IK_HD SearchPlan disc_search_plan(const ArmConst &A, const R2ikCtlParams &par, const Solve &S, const Reach &rc) {
+  SearchPlan P = disc_search_plan(par, rc.i0, rc.i1);
+  P.T = make_elbow_test(A, S);
+  return P;
+}
+
+// The arg-min of the K-sample search (utl:376-390) from a plan: search_analytic, or the exhaustive scan where its atan2
+// arguments are out of range.  false: no valid sample (theta untouched).
+R2IK_HD bool disc_search(const SearchPlan &P, int nb, double &theta) {
+  double best;
+  int best_k;
+  if (!search_analytic(P, nb, best, best_k)) search_strided(P, nb, 0, 1, best, best_k);
+  const bool found = best < INFINITY;
+  if (found) theta = linspace_value(P.L, best_k);
+  return found;
 }
 
 // ---------------------------------------------------------------------------------------

@@ -828,6 +828,12 @@ R2IK_HD bool is_elbow_ok(const ArmConst &A, const double E[3]) {
   return ok;
 }
 
+// sik:697-718: get_joints takes the make_elbow_projection branch for this elbow position.  (The reference then returns
+// the elbow as a 3-vector instead of get_elbow_position's homogeneous [x, y, z, 1], sik:714, :863.)
+R2IK_HD bool elbow_projection_fires(const ArmConst &A, const double E[3]) {
+  return E[2] > (E[0] - A.es[0]) * A.sing_coeff + A.es[2] - A.sing_offset;
+}
+
 // 2-D rotation helpers: the reference's elementary frame changes (sik:758-837)
 struct P3 { double x, y, z; };
 R2IK_HD void rot_y(P3 &p, double c, double s) {  // R_y(a) with c = cos a, s = sin a
@@ -863,7 +869,7 @@ R2IK_HD bool get_joints_impl(const ArmConst &A, Solve &S, double ct, double st, 
                              double E[3]) {
   bool degenerate = false;
   elbow_position_cs(S, ct, st, E);
-  if (E[2] > (E[0] - A.es[0]) * A.sing_coeff + A.es[2] - A.sing_offset) {
+  if (elbow_projection_fires(A, E)) {
     // sik:647-682 make_elbow_projection with the plane constants hoisted to the host
     double dist = (E[0] - A.plP[0]) * A.plV[0] + (E[1] - A.plP[1]) * A.plV[1] + (E[2] - A.plP[2]) * A.plV[2];
     double vc[3] = {E[0] - dist * A.plV[0] - A.plC[0], E[1] - dist * A.plV[1] - A.plC[1], E[2] - dist * A.plV[2] - A.plC[2]};
@@ -1054,6 +1060,126 @@ R2IK_HD bool rotation_from_mat4(const double *M, bool snap, double R[9]) {
   bool ok = rotation_from_mat3_literal(mm, RR);
   for (int k = 0; k < 9; ++k) R[k] = RR[k];
   return ok;
+}
+
+// Doubles per row of a pose buffer
+R2IK_HD constexpr int pose_stride(int kind) { return kind == R2IK_POSE_EULER6 ? 6 : kind == R2IK_POSE_MAT34 ? 12 : 16; }
+
+// Two doubles at a 16-byte aligned address (pose buffers: checked by the C entry points): one 128-bit read-only load on
+// the device
+R2IK_HD void load2(const double *p, double &a, double &b) {
+#if defined(__CUDA_ARCH__)
+  const double2 v = __ldg(reinterpret_cast<const double2 *>(p));
+  a = v.x; b = v.y;
+#else
+  a = p[0]; b = p[1];
+#endif
+}
+
+// 3x4 top of a row-major 4x4 (the last row is never read): 6 x 128-bit loads
+R2IK_HD void load_mat4(const double *M, double m[16]) {
+#pragma unroll
+  for (int r = 0; r < 3; ++r) {
+    load2(M + 4 * r, m[4 * r], m[4 * r + 1]);
+    load2(M + 4 * r + 2, m[4 * r + 2], m[4 * r + 3]);
+  }
+  m[12] = 0.0; m[13] = 0.0; m[14] = 0.0; m[15] = 1.0;
+}
+
+// Goal position + goal rotation matrix of one pose row.  false <=> invalid rotation (det <= 0).  MAT34 rows are the
+// 3x4 top of the matrix, 12 doubles per pose: every byte that crosses HBM (and PCIe) is used.
+template <int KIND>
+R2IK_HD bool load_pose(const double *row, bool snap, double pos[3], double R[9]) {
+  if (KIND == R2IK_POSE_EULER6) {
+    double e[3];
+    load2(row, pos[0], pos[1]);
+    load2(row + 2, pos[2], e[0]);
+    load2(row + 4, e[1], e[2]);
+    rot_from_euler_xyz(e[0], e[1], e[2], R);
+    return true;
+  }
+  double m[16];
+  load_mat4(row, m);
+  pos[0] = m[3]; pos[1] = m[7]; pos[2] = m[11];
+  return rotation_from_mat4(m, snap, R);
+}
+
+// ---------------------------------------------------------------------------------------
+// Per-pose bodies of the SymbolicIK kernels (r2ik_kernels.cu; tests/hostsim loops over the same functions)
+// ---------------------------------------------------------------------------------------
+// K1, solve: is_reachable on a pose row (INVALID_ROTATION with a NaN interval for det <= 0).
+template <int KIND>
+R2IK_HD Reach symik_reach(const ArmConst &A, const double *row, Solve &S) {
+  double pos[3];
+  Reach rc;
+  rc.state = R2IK_STATE_INVALID_ROTATION; rc.i0 = NAN; rc.i1 = NAN;
+  if (load_pose<KIND>(row, false, pos, S.R)) rc = is_reachable_R<false>(A, pos, S);
+  return rc;
+}
+
+// K1, joints: get_joints at *theta, or without theta at theta_interval[0] (its cos / sin come with the interval); NaN
+// for a pose that is not reachable.
+R2IK_HD void symik_joints(const ArmConst &A, Solve &S, const Reach &rc, const double *theta, double prev0, double prev2,
+                          double j[7], double E[3]) {
+  if (rc.state == R2IK_STATE_REACHABLE) {
+    double ct = rc.c0, st = rc.s0;
+    if (theta) sincos_any(*theta, st, ct);
+    get_joints_cs(A, S, ct, st, prev0, prev2, j, E);
+  } else {
+#pragma unroll
+    for (int k = 0; k < 7; ++k) j[k] = NAN;
+    E[0] = NAN; E[1] = NAN; E[2] = NAN;
+  }
+}
+
+// K1b: is_reachable_no_limits + get_joints(*theta, prev[0], prev[2]) (prev may be null: zeros; they only matter at the
+// exact singularities, sik:751, 782).  NaN without an elbow circle or for an invalid rotation.  Returns whether the
+// elbow projection fires at theta.
+template <int KIND>
+R2IK_HD bool symik_no_limits(const ArmConst &A, const double *row, const double *theta, const double *prev, double j[7],
+                             double E[3]) {
+  double pos[3];
+  Solve S;
+  bool ok = load_pose<KIND>(row, false, pos, S.R);
+  if (ok) ok = is_reachable_R<true>(A, pos, S).state == R2IK_STATE_REACHABLE;
+  bool proj = false;
+  if (ok) {
+    double prev0 = 0.0, prev2 = 0.0;
+    if (prev) { prev0 = prev[0]; prev2 = prev[2]; }
+    double st, ct, Ep[3];
+    sincos_any(*theta, st, ct);
+    elbow_position_cs(S, ct, st, Ep);
+    proj = elbow_projection_fires(A, Ep);
+    get_joints_cs(A, S, ct, st, prev0, prev2, j, E);
+  } else {
+    for (int k = 0; k < 7; ++k) j[k] = NAN;
+    E[0] = NAN; E[1] = NAN; E[2] = NAN;
+  }
+  return proj;
+}
+
+// K1b: the elbow circle is_reachable (NO_LIMITS = false) or is_reachable_no_limits (true) stores for a pose row.  The
+// reference stores the circle as soon as it exists (sik:197), i.e. also when the wrist limit then rejects the pose.
+// false: no circle.
+template <int KIND, bool NO_LIMITS>
+R2IK_HD bool pose_elbow_circle(const ArmConst &A, const double *row, Solve &S) {
+  double pos[3];
+  bool ok = load_pose<KIND>(row, false, pos, S.R);
+  if (ok) {
+    const int st = is_reachable_R<NO_LIMITS>(A, pos, S).state;
+    ok = st == R2IK_STATE_REACHABLE || (!NO_LIMITS && st == R2IK_STATE_LIMITED_BY_WRIST);
+  }
+  return ok;
+}
+
+// get_elbow_position(*theta) on that circle (NaN without one).  Returns whether the elbow projection fires there.
+R2IK_HD bool elbow_on_circle(const ArmConst &A, const Solve &S, bool circle, const double *theta, double E[3]) {
+  E[0] = NAN; E[1] = NAN; E[2] = NAN;
+  if (!circle) return false;
+  double st, ct;
+  sincos_any(*theta, st, ct);
+  elbow_position_cs(S, ct, st, E);
+  return elbow_projection_fires(A, E);
 }
 
 }  // namespace r2ik

@@ -520,6 +520,20 @@ R2IK_HD int reach_flag_mixed(const ArmConst &A64, const ArmConstF &A, const doub
   return R2IK_STATE_REACHABLE;
 }
 
+// The state of one (voxel p, orientation) pair: reach_flag_mixed, and where it is too close to call in FP32 (esc) the
+// FP64 flag solve on the orientation's xyz Euler angles e.
+R2IK_HD int reach_pair(const ArmConst &A64, const ArmConstF &A, const double ps[3], double px, double py, double pz,
+                       const OriConst &O, const double *e, bool &esc) {
+  int st = reach_flag_mixed(A64, A, ps, px, O, esc);
+  if (esc) {
+    Solve S;
+    S.p[0] = px; S.p[1] = py; S.p[2] = pz;
+    rot_from_euler_xyz(e[0], e[1], e[2], S.R);
+    st = solve_core<false, true>(A64, S).state;
+  }
+  return st;
+}
+
 // ---------------------------------------------------------------------------------------
 // per-pose bodies of K1-f32
 // ---------------------------------------------------------------------------------------

@@ -36,13 +36,80 @@ static_assert(sizeof(DiscHeader) == 256, "DiscHeader is two 128-byte lines");
 
 constexpr uint32_t kDiscLiteral = 0x80000000u;   // flag bit of a list entry (n < 2^31)
 
+R2IK_HD size_t disc_ws_bytes(int64_t n) { return sizeof(DiscHeader) + (size_t)n * (64 + 8 + 4 + 4); }
+
+// The search plan of a listed pose, 8 doubles (64 bytes, 16-byte aligned): i0, i1, A1, B1, C1, A2, B2, C2
+R2IK_HD void disc_plan_pack(double *p, const ArmConst &A, const Solve &S, double i0, double i1) {
+  const ElbowTest T = make_elbow_test(A, S);
+#if defined(__CUDA_ARCH__)
+  double2 *q = reinterpret_cast<double2 *>(p);
+  q[0] = make_double2(i0, i1);
+  q[1] = make_double2(T.A1, T.B1);
+  q[2] = make_double2(T.C1, T.A2);
+  q[3] = make_double2(T.B2, T.C2);
+#else
+  p[0] = i0; p[1] = i1; p[2] = T.A1; p[3] = T.B1; p[4] = T.C1; p[5] = T.A2; p[6] = T.B2; p[7] = T.C2;
+#endif
+}
+
+R2IK_HD SearchPlan disc_plan_unpack(const R2ikCtlParams &par, const double *p) {
+  double q[8];
+#if defined(__CUDA_ARCH__)
+  const double2 *p2 = reinterpret_cast<const double2 *>(p);
+  const double2 q0 = p2[0], q1 = p2[1], q2 = p2[2], q3 = p2[3];
+  q[0] = q0.x; q[1] = q0.y; q[2] = q1.x; q[3] = q1.y; q[4] = q2.x; q[5] = q2.y; q[6] = q3.x; q[7] = q3.y;
+#else
+  for (int k = 0; k < 8; ++k) q[k] = p[k];
+#endif
+  SearchPlan P = disc_search_plan(par, q[0], q[1]);
+  P.T.A1 = q[2]; P.T.B1 = q[3]; P.T.C1 = q[4]; P.T.A2 = q[5]; P.T.B2 = q[6]; P.T.C2 = q[7];
+  return P;
+}
+
+// Finish a listed pose at its theta.  The elbow circle is all get_joints needs of the solve: the circle linking (a
+// quarter of is_reachable) is not redone, except for the rare pose whose solve took the literal instantiation (its S is
+// that instantiation's).  Returns the emergency bits.
+R2IK_HD int disc_finish_listed(const ArmConst &A, const R2ikCtlParams &par, const double *row, bool literal, double theta,
+                               const double prev[7], double j[7]) {
+  Solve S;
+  double pos[3];
+  load_pose<R2IK_POSE_MAT4>(row, true, pos, S.R);       // valid and reachable: k_disc_classify listed it
+  if (literal) is_reachable_R<false>(A, pos, S);
+  else circle_of_reachable(A, pos, S);
+  return discrete_finish(A, par, S, true, theta, prev, prev, j);
+}
+
+// Empty lists, and the result every pose without a valid theta shares (current_joints through safety_checks: ctl:454-462
+// with found = false)
+R2IK_HD void disc_header_init(DiscHeader *hdr, const R2ikCtlParams &par, const double *prev_joints, const double *current_joints) {
+  double prev[7], j[7];
+  for (int k = 0; k < 7; ++k) { prev[k] = prev_joints[k]; j[k] = current_joints[k]; }
+  const int bits = safety_checks(j, prev, par.orbita3d_max_angle);
+  for (int k = 0; k < 7; ++k) hdr->nf_joints[k] = j[k];
+  hdr->nf_bits = bits;
+  hdr->n_search = 0;
+  hdr->n_finish = 0;
+}
+
+// the result of a pose without a valid theta (or NaN joints for an invalid rotation)
+R2IK_HD void disc_store_final(const DiscHeader *hdr, int64_t i, int st, double *__restrict__ joints,
+                              uint8_t *__restrict__ reachable, uint8_t *__restrict__ state, uint8_t *__restrict__ emergency) {
+  const bool invalid = st == R2IK_STATE_INVALID_ROTATION;
+#pragma unroll
+  for (int k = 0; k < 7; ++k) joints[7 * i + k] = invalid ? NAN : hdr->nf_joints[k];
+  reachable[i] = 0;
+  state[i] = (uint8_t)st;
+  if (emergency) emergency[i] = invalid ? 0 : (uint8_t)hdr->nf_bits;
+}
+
+#if defined(__CUDACC__)
+
 struct DiscWs {
   DiscHeader *hdr;
-  double *plan;           // 8 doubles per search-list entry: i0, i1, A1, B1, C1, A2, B2, C2
+  double *plan;           // 8 doubles per search-list entry (disc_plan_pack)
   double *finish_theta;
   uint32_t *search_idx, *finish_idx;
 };
-inline __host__ __device__ size_t disc_ws_bytes(int64_t n) { return sizeof(DiscHeader) + (size_t)n * (64 + 8 + 4 + 4); }
 inline __host__ DiscWs disc_ws_carve(void *ws, int64_t n) {
   DiscWs w;
   char *p = static_cast<char *>(ws);
@@ -53,8 +120,6 @@ inline __host__ DiscWs disc_ws_carve(void *ws, int64_t n) {
   w.finish_idx = reinterpret_cast<uint32_t *>(p);
   return w;
 }
-
-#if defined(__CUDACC__)
 
 // Programmatic dependent launch: the four kernels of a call are chained on one stream, each launched with
 // cudaLaunchAttributeProgrammaticStreamSerialization.  A kernel lets its successor's blocks be scheduled early
@@ -86,34 +151,13 @@ __device__ __forceinline__ unsigned disc_append2(bool p0, bool p1, unsigned *cou
   return slot;          // one call per block (the shared counters are not reused)
 }
 
-// the result of a pose without a valid theta (or NaN joints for an invalid rotation block)
-__device__ __forceinline__ void disc_store_final(const DiscHeader *hdr, int64_t i, int st, double *__restrict__ joints,
-                                                 uint8_t *__restrict__ reachable, uint8_t *__restrict__ state,
-                                                 uint8_t *__restrict__ emergency) {
-  const bool invalid = st == R2IK_STATE_INVALID_ROTATION;
-#pragma unroll
-  for (int k = 0; k < 7; ++k) joints[7 * i + k] = invalid ? NAN : hdr->nf_joints[k];
-  reachable[i] = 0;
-  state[i] = (uint8_t)st;
-  if (emergency) emergency[i] = invalid ? 0 : (uint8_t)hdr->nf_bits;
-}
-
 __global__ void k_disc_consts(const __grid_constant__ R2ikCtlParams par, const double *__restrict__ prev_joints,
                               const double *__restrict__ current_joints, DiscHeader *hdr) {
   disc_launch_dependents();
   if (threadIdx.x || blockIdx.x) return;
-  double prev[7], j[7];
-  for (int k = 0; k < 7; ++k) { prev[k] = prev_joints[k]; j[k] = current_joints[k]; }
-  const int bits = safety_checks(j, prev, par.orbita3d_max_angle);
-  for (int k = 0; k < 7; ++k) hdr->nf_joints[k] = j[k];
-  hdr->nf_bits = bits;
-  hdr->n_search = 0;
-  hdr->n_finish = 0;
+  disc_header_init(hdr, par, prev_joints, current_joints);
 }
 
-#ifndef R2IK_K2C_CIRCLE_ONLY
-#define R2IK_K2C_CIRCLE_ONLY 1
-#endif
 #ifndef R2IK_K2C_CLASSIFY_MINBLOCKS
 #define R2IK_K2C_CLASSIFY_MINBLOCKS 6
 #endif
@@ -133,38 +177,25 @@ k_disc_classify(const __grid_constant__ ArmConst A, const __grid_constant__ R2ik
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const bool active = i < n;
   Solve S;
-  int st = R2IK_STATE_INVALID_ROTATION;
+  Reach rc;
+  rc.state = R2IK_STATE_INVALID_ROTATION;
   bool shortcut = false, need_search = false;
-  double i0 = 0.0, i1 = 0.0;
   uint32_t tag = (uint32_t)i;      // list entry: pose index, bit 31 = the solve took the literal instantiation
   if (active) {
-    double pos[3];
-    if (load_pose<R2IK_POSE_MAT4>(M, i, true, pos, S.R)) {
-      Reach rc = is_reachable_R<false>(A, pos, S);
-      st = rc.state; i0 = rc.i0; i1 = rc.i1;
-      if (rc.literal) tag |= kDiscLiteral;
-      if (st == R2IK_STATE_REACHABLE) {
-        shortcut = preferred_theta_works(A, S, i0, i1, par.preferred_theta);
-        need_search = !shortcut;
-      }
-    }
+    disc_classify(A, par, M + 16 * i, S, rc, shortcut, need_search);
+    if (rc.literal) tag |= kDiscLiteral;
   }
   disc_wait_predecessor();      // k_disc_consts: the counters are reset, the shared result is there (the poses are the caller's)
   const unsigned slot = disc_append2(need_search, shortcut, &hdr->n_search, &hdr->n_finish);
   if (need_search) {
-    const ElbowTest T = make_elbow_test(A, S);
     search_idx[slot] = tag;
-    double2 *p = reinterpret_cast<double2 *>(plan + 8 * (size_t)slot);
-    p[0] = make_double2(i0, i1);
-    p[1] = make_double2(T.A1, T.B1);
-    p[2] = make_double2(T.C1, T.A2);
-    p[3] = make_double2(T.B2, T.C2);
+    disc_plan_pack(plan + 8 * (size_t)slot, A, S, rc.i0, rc.i1);
   }
   if (shortcut) {
     finish_idx[slot] = tag;
     finish_theta[slot] = par.preferred_theta;
   }
-  if (active && !need_search && !shortcut) disc_store_final(hdr, i, st, joints, reachable, state, emergency);
+  if (active && !need_search && !shortcut) disc_store_final(hdr, i, rc.state, joints, reachable, state, emergency);
 }
 
 __global__ void __launch_bounds__(R2IK_BLOCK, R2IK_K2C_SEARCH_MINBLOCKS)
@@ -184,20 +215,7 @@ k_disc_search(const __grid_constant__ R2ikCtlParams par, DiscHeader *hdr, const 
   uint32_t i = 0;
   if (active) {
     i = search_idx[k];
-    const double2 *p = reinterpret_cast<const double2 *>(plan + 8 * (size_t)k);
-    const double2 q0 = p[0], q1 = p[1], q2 = p[2], q3 = p[3];
-    SearchPlan P;
-    P.preferred_theta = par.preferred_theta;
-    double start, stop;
-    search_range(q0.x, q0.y, start, stop);
-    P.L = make_linspace(start, stop, par.nb_search_points);
-    P.T.A1 = q1.x; P.T.B1 = q1.y; P.T.C1 = q2.x; P.T.A2 = q2.y; P.T.B2 = q3.x; P.T.C2 = q3.y;
-    double best;
-    int best_k;
-    if (!search_analytic(P, par.nb_search_points, best, best_k))
-      search_strided(P, par.nb_search_points, 0, 1, best, best_k);     // out-of-range magnitudes: scan
-    found = best < INFINITY;
-    if (found) theta = linspace_value(P.L, best_k);
+    found = disc_search(disc_plan_unpack(par, plan + 8 * (size_t)k), par.nb_search_points, theta);
   }
   const unsigned kf = disc_append2(false, found, &hdr->n_finish, &hdr->n_finish);
   if (found) {
@@ -225,15 +243,8 @@ k_disc_finish(const __grid_constant__ ArmConst A, const __grid_constant__ R2ikCt
   for (int q = 0; q < 7; ++q) prev[q] = prev_joints[q];
   const uint32_t tag = finish_idx[k];
   const int64_t i = tag & ~kDiscLiteral;
-  const double theta = finish_theta[k];
-  Solve S;
-  double pos[3], j[7];
-  load_pose<R2IK_POSE_MAT4>(M, i, true, pos, S.R);       // valid and reachable: k_disc_classify listed it
-  // the elbow circle is all get_joints needs of the solve: the circle linking (a quarter of is_reachable) is not redone,
-  // except for the rare pose whose solve took the literal instantiation (its S is that instantiation's)
-  if (!R2IK_K2C_CIRCLE_ONLY || (tag & kDiscLiteral)) is_reachable_R<false>(A, pos, S);
-  else circle_of_reachable(A, pos, S);
-  const int bits = discrete_finish(A, par, S, true, theta, prev, prev, j);
+  double j[7];
+  const int bits = disc_finish_listed(A, par, M + 16 * i, (tag & kDiscLiteral) != 0, finish_theta[k], prev, j);
 #pragma unroll
   for (int q = 0; q < 7; ++q) joints[7 * i + q] = j[q];
   reachable[i] = 1;

@@ -33,149 +33,39 @@ using namespace r2ik;
 #ifndef R2IK_K1_MINBLOCKS
 #define R2IK_K1_MINBLOCKS 4   // resident blocks / SM the register allocation of K1 is held to
 #endif
-#ifndef R2IK_K1_STAGED
-#define R2IK_K1_STAGED 0      // 1: K1's float outputs leave through shared memory as 128-bit row-contiguous stores
-#endif
-#ifndef R2IK_K1_PDL
-#define R2IK_K1_PDL 1         // K1 launches are programmatic dependents of what precedes them on the stream: back-to-back launches (two arms, pipeline chunks) overlap their launch latency, 0.1305 -> 0.1250 ms per 2 x 1M poses
-#endif
-
-// ---------------------------------------------------------------------------------------
-// vectorised global memory helpers
-// ---------------------------------------------------------------------------------------
-// 128-bit read-only load: pose buffers must be 16-byte aligned (checked by the C entry points)
-__device__ __forceinline__ double2 ldg2(const double *p) { return __ldg(reinterpret_cast<const double2 *>(p)); }
-
-// 3x4 top of a row-major 4x4 (the last row is never read): 6 x 128-bit loads
-__device__ __forceinline__ void load_mat4(const double *__restrict__ M, double m[16]) {
-#pragma unroll
-  for (int r = 0; r < 3; ++r) {
-    double2 a = ldg2(M + 4 * r), b = ldg2(M + 4 * r + 2);
-    m[4 * r] = a.x; m[4 * r + 1] = a.y; m[4 * r + 2] = b.x; m[4 * r + 3] = b.y;
-  }
-  m[12] = 0.0; m[13] = 0.0; m[14] = 0.0; m[15] = 1.0;
-}
-
-// Goal position + goal rotation matrix of pose i.  false <=> invalid rotation (det <= 0).
-template <int KIND>
-__device__ __forceinline__ bool load_pose(const double *__restrict__ poses, int64_t i, bool snap, double pos[3], double R[9]) {
-  if (KIND == R2IK_POSE_EULER6) {
-    const double *p = poses + 6 * i;
-    double2 a = ldg2(p), b = ldg2(p + 2), c = ldg2(p + 4);
-    pos[0] = a.x; pos[1] = a.y; pos[2] = b.x;
-    rot_from_euler_xyz(b.y, c.x, c.y, R);
-    return true;
-  } else if (KIND == R2IK_POSE_MAT34) {
-    // the 3x4 top of the matrix, 12 doubles per pose: every byte that crosses HBM (and PCIe) is used
-    double m[16];
-    const double *p = poses + 12 * i;
-#pragma unroll
-    for (int r = 0; r < 3; ++r) {
-      double2 a = ldg2(p + 4 * r), b = ldg2(p + 4 * r + 2);
-      m[4 * r] = a.x; m[4 * r + 1] = a.y; m[4 * r + 2] = b.x; m[4 * r + 3] = b.y;
-    }
-    m[12] = 0.0; m[13] = 0.0; m[14] = 0.0; m[15] = 1.0;
-    pos[0] = m[3]; pos[1] = m[7]; pos[2] = m[11];
-    return rotation_from_mat4(m, snap, R);
-  } else {
-    double m[16];
-    load_mat4(poses + 16 * i, m);
-    pos[0] = m[3]; pos[1] = m[7]; pos[2] = m[11];
-    return rotation_from_mat4(m, snap, R);
-  }
-}
-
-__device__ __forceinline__ void store_nan(double *p, int n) {
-  for (int k = 0; k < n; ++k) p[k] = NAN;
-}
 
 // ---------------------------------------------------------------------------------------
 // K1: SymbolicIK.is_reachable + theta_to_joints
 // ---------------------------------------------------------------------------------------
-// STAGED = true: the three float outputs of a warp's 32 poses (7 + 3 + 2 doubles each) are transposed through 3 KB of
-// shared memory and leave as 128-bit row-contiguous stores (every sector written once, by one request) instead of 12
-// scalar stores of stride 56 / 24 / 16 bytes.  Needs 16-byte aligned output arrays (the launcher checks).
-template <int KIND, bool STAGED>
+// Launched as a programmatic dependent of what precedes it on the stream (launch_pdl): back-to-back launches (two arms,
+// pipeline chunks) overlap their launch latency, 0.1305 -> 0.1250 ms per 2 x 1M poses.
+template <int KIND>
 __global__ void __launch_bounds__(R2IK_BLOCK, R2IK_K1_MINBLOCKS)
 k_symik_solve(const __grid_constant__ ArmConst A, const double *__restrict__ poses, const double *__restrict__ theta,
               const double *__restrict__ prev_joints, int64_t n, uint8_t *__restrict__ reachable,
               uint8_t *__restrict__ state, double *__restrict__ interval, double *__restrict__ joints,
               double *__restrict__ elbow) {
-  __shared__ double s_stage[STAGED ? R2IK_BLOCK / 32 : 1][STAGED ? 32 * 12 : 1];
-#if R2IK_K1_PDL
   // the next kernel on the stream may be scheduled as soon as every block of this one has started; this one touches
   // memory only once its own predecessor has completed
   asm volatile("griddepcontrol.launch_dependents;");
   asm volatile("griddepcontrol.wait;" ::: "memory");
-#endif
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const bool active = i < n;
-  if (!STAGED && !active) return;
+  if (i >= n) return;
   double prev0 = 0.0, prev2 = 0.0;
   if (prev_joints) { prev0 = prev_joints[0]; prev2 = prev_joints[2]; }
-  double pos[3];
   Solve S;
-  Reach rc;
-  rc.state = R2IK_STATE_INVALID_ROTATION; rc.i0 = NAN; rc.i1 = NAN;
-  if (active && load_pose<KIND>(poses, i, false, pos, S.R)) rc = is_reachable_R<false>(A, pos, S);
-  bool ok = active && rc.state == R2IK_STATE_REACHABLE;
-  if (active) {
-    if (reachable) reachable[i] = ok ? 1 : 0;   // nullable: state == R2IK_STATE_REACHABLE says the same (lean host record)
-    state[i] = (uint8_t)rc.state;
-  }
-  if (!STAGED) {
-    if (interval) { interval[2 * i] = rc.i0; interval[2 * i + 1] = rc.i1; }
-    if (!joints && !elbow) return;
-  }
+  const Reach rc = symik_reach<KIND>(A, poses + pose_stride(KIND) * i, S);
+  if (reachable) reachable[i] = rc.state == R2IK_STATE_REACHABLE ? 1 : 0;   // nullable: state == R2IK_STATE_REACHABLE says the same (lean host record)
+  state[i] = (uint8_t)rc.state;
+  if (interval) { interval[2 * i] = rc.i0; interval[2 * i + 1] = rc.i1; }
+  if (!joints && !elbow) return;
   double j[7], E[3];
-  if (ok && (joints || elbow)) {
-    double ct = rc.c0, st = rc.s0;   // theta_interval[0]: its cos / sin come with the interval
-    if (theta) sincos_any(theta[i], st, ct);
-    get_joints_cs(A, S, ct, st, prev0, prev2, j, E);
-  } else {
-#pragma unroll
-    for (int k = 0; k < 7; ++k) j[k] = NAN;
-    E[0] = NAN; E[1] = NAN; E[2] = NAN;
-  }
-  if (!STAGED) {
-    if (joints) {
-#pragma unroll
-      for (int k = 0; k < 7; ++k) joints[7 * i + k] = j[k];
-    }
-    if (elbow) { elbow[3 * i] = E[0]; elbow[3 * i + 1] = E[1]; elbow[3 * i + 2] = E[2]; }
-    return;
-  }
-  // ---- staged stores: [0, 224) joints, [224, 320) elbow, [320, 384) interval of the warp's 32 poses
-  const int lane = threadIdx.x & 31;
-  double *sw = s_stage[STAGED ? threadIdx.x >> 5 : 0];
-#pragma unroll
-  for (int k = 0; k < 7; ++k) sw[7 * lane + k] = j[k];
-  sw[224 + 3 * lane] = E[0]; sw[224 + 3 * lane + 1] = E[1]; sw[224 + 3 * lane + 2] = E[2];
-  sw[320 + 2 * lane] = rc.i0; sw[320 + 2 * lane + 1] = rc.i1;
-  __syncwarp();
-  const int64_t i0 = i - lane;                                  // first pose of the warp
-  const int64_t left = n - i0;
-  const int cnt = left < 32 ? (int)left : 32;                   // poses of this warp inside the batch (> 0 for a launched warp)
-  if (cnt <= 0) return;
-  const double2 *s2 = reinterpret_cast<const double2 *>(sw);
+  symik_joints(A, S, rc, theta ? theta + i : nullptr, prev0, prev2, j, E);
   if (joints) {
-    double2 *g = reinterpret_cast<double2 *>(joints + 7 * i0);
-    const int n2 = (7 * cnt) >> 1;
 #pragma unroll
-    for (int q = 0; q < 4; ++q) { const int e = lane + 32 * q; if (e < n2) g[e] = s2[e]; }
-    if (((7 * cnt) & 1) && lane == 0) joints[7 * i0 + 7 * cnt - 1] = sw[7 * cnt - 1];
+    for (int k = 0; k < 7; ++k) joints[7 * i + k] = j[k];
   }
-  if (elbow) {
-    double2 *g = reinterpret_cast<double2 *>(elbow + 3 * i0);
-    const int n2 = (3 * cnt) >> 1;
-#pragma unroll
-    for (int q = 0; q < 2; ++q) { const int e = lane + 32 * q; if (e < n2) g[e] = s2[112 + e]; }
-    if (((3 * cnt) & 1) && lane == 0) elbow[3 * i0 + 3 * cnt - 1] = sw[224 + 3 * cnt - 1];
-  }
-  if (interval) {
-    double2 *g = reinterpret_cast<double2 *>(interval + 2 * i0);
-    if (lane < cnt) g[lane] = s2[160 + lane];
-  }
+  if (elbow) { elbow[3 * i] = E[0]; elbow[3 * i + 1] = E[1]; elbow[3 * i + 2] = E[2]; }
 }
 
 // ---------------------------------------------------------------------------------------
@@ -284,14 +174,6 @@ k_symik_escalated_f32(const __grid_constant__ ArmConst A64, const float *__restr
   }
 }
 
-// sik:697-718: does get_joints(cos theta, sin theta) take the make_elbow_projection branch on the solved pose?  (The
-// reference then returns the elbow as a 3-vector instead of get_elbow_position's homogeneous [x, y, z, 1], sik:714, :863.)
-__device__ __forceinline__ bool elbow_projection_fires(const ArmConst &A, const Solve &S, double ct, double st) {
-  double E[3];
-  elbow_position_cs(S, ct, st, E);
-  return E[2] > (E[0] - A.es[0]) * A.sing_coeff + A.es[2] - A.sing_offset;
-}
-
 template <int KIND>
 __global__ void __launch_bounds__(R2IK_BLOCK)
 k_symik_no_limits(const __grid_constant__ ArmConst A, const double *__restrict__ poses, const double *__restrict__ theta,
@@ -299,51 +181,25 @@ k_symik_no_limits(const __grid_constant__ ArmConst A, const double *__restrict__
                   double *__restrict__ elbow, uint8_t *__restrict__ projected) {
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  double pos[3], j[7], E[3];
-  Solve S;
-  bool ok = load_pose<KIND>(poses, i, false, pos, S.R);
-  if (ok) ok = is_reachable_R<true>(A, pos, S).state == R2IK_STATE_REACHABLE;
-  bool proj = false;
-  if (ok) {
-    double prev0 = 0.0, prev2 = 0.0;   // previous_joints only matter at the exact singularities (sik:751, 782)
-    if (prev_joints) { prev0 = prev_joints[(size_t)prev_stride * i]; prev2 = prev_joints[(size_t)prev_stride * i + 2]; }
-    double st, ct;
-    sincos_any(theta[i], st, ct);
-    proj = elbow_projection_fires(A, S, ct, st);
-    get_joints_cs(A, S, ct, st, prev0, prev2, j, E);
-  } else {
-    for (int k = 0; k < 7; ++k) j[k] = NAN;
-    E[0] = NAN; E[1] = NAN; E[2] = NAN;
-  }
+  double j[7], E[3];
+  const bool proj = symik_no_limits<KIND>(A, poses + pose_stride(KIND) * i, theta + i,
+                                          prev_joints ? prev_joints + (size_t)prev_stride * i : nullptr, j, E);
   for (int k = 0; k < 7; ++k) joints[7 * i + k] = j[k];
   if (elbow) { elbow[3 * i] = E[0]; elbow[3 * i + 1] = E[1]; elbow[3 * i + 2] = E[2]; }
   if (projected) projected[i] = proj ? 1 : 0;
 }
 
-// get_elbow_position(thetas[i][k]) on the circle is_reachable (NO_LIMITS = false) or is_reachable_no_limits (true) stores.
-// The reference stores the circle as soon as it exists (sik:197), i.e. also when the wrist limit then rejects the pose.
 template <int KIND, bool NO_LIMITS>
 __global__ void __launch_bounds__(R2IK_BLOCK)
 k_elbow_positions(const __grid_constant__ ArmConst A, const double *__restrict__ poses, const double *__restrict__ thetas,
                   int K, int64_t n, double *__restrict__ elbows, uint8_t *__restrict__ projected) {
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  double pos[3];
   Solve S;
-  bool ok = load_pose<KIND>(poses, i, false, pos, S.R);
-  if (ok) {
-    const int st = is_reachable_R<NO_LIMITS>(A, pos, S).state;
-    ok = st == R2IK_STATE_REACHABLE || (!NO_LIMITS && st == R2IK_STATE_LIMITED_BY_WRIST);
-  }
+  const bool circle = pose_elbow_circle<KIND, NO_LIMITS>(A, poses + pose_stride(KIND) * i, S);
   for (int k = 0; k < K; ++k) {
-    double E[3] = {NAN, NAN, NAN};
-    bool proj = false;
-    if (ok) {
-      double st, ct;
-      sincos_any(thetas[(size_t)i * K + k], st, ct);
-      elbow_position_cs(S, ct, st, E);
-      proj = E[2] > (E[0] - A.es[0]) * A.sing_coeff + A.es[2] - A.sing_offset;
-    }
+    double E[3];
+    const bool proj = elbow_on_circle(A, S, circle, thetas + ((size_t)i * K + k), E);
     double *o = elbows + ((size_t)i * K + k) * 3;
     o[0] = E[0]; o[1] = E[1]; o[2] = E[2];
     if (projected) projected[(size_t)i * K + k] = proj ? 1 : 0;
@@ -375,7 +231,7 @@ __device__ __forceinline__ void scalar_body(const ArmConst &A, const R2ikScalarQ
     if (q.has_theta) sincos_any(q.theta, st, ct);
     elbow_position_cs(S, ct, st, r.elbow_on_circle);
     if (r.reachable) {
-      r.projected = elbow_projection_fires(A, S, ct, st) ? 1 : 0;
+      r.projected = elbow_projection_fires(A, r.elbow_on_circle) ? 1 : 0;
       get_joints_cs(A, S, ct, st, q.previous_joints[0], q.previous_joints[2], r.joints, r.elbow);
       for (int k = 0; k < 3; ++k) { r.goal_position[k] = S.p[k]; r.wrist_position[k] = S.w[k]; }
     }
@@ -398,19 +254,13 @@ k_symik_scalar(const __grid_constant__ ArmConst A, const __grid_constant__ R2ikS
   *out = r;
 }
 
-// ControlIK.__init__'s seed of previous_theta (ctl:142-159): is_reachable_no_limits on the current pose (identity snap of
-// ctl:142), then the constructor's form of the ternary search.  One thread; arguments by value; result to any
+// ControlIK.__init__'s seed of previous_theta (ctl_ctor_theta).  One thread; arguments by value; result to any
 // device-accessible address.
 struct CtorThetaArgs { double rows[49]; double current_pose[16]; double preferred_theta; int n_rows; int pad; };
 __global__ void __launch_bounds__(32)
 k_ctl_ctor_theta(const __grid_constant__ ArmConst A, const __grid_constant__ CtorThetaArgs a, double *__restrict__ out) {
   if (threadIdx.x != 0 || blockIdx.x != 0) return;
-  Solve S;
-  const double cpos[3] = {a.current_pose[3], a.current_pose[7], a.current_pose[11]};
-  double theta = NAN;
-  if (rotation_from_mat4(a.current_pose, true, S.R) && is_reachable_R<true>(A, cpos, S).state == R2IK_STATE_REACHABLE)
-    theta = ctor_previous_theta(A, S, a.rows, a.n_rows, a.preferred_theta);
-  out[0] = theta;
+  out[0] = ctl_ctor_theta(A, a.current_pose, a.rows, a.n_rows, a.preferred_theta);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -455,25 +305,12 @@ k_ctl_discrete_scan(const __grid_constant__ ArmConst A, const __grid_constant__ 
   double theta = 0.0;
   const int nb = par.nb_search_points;
   SearchPlan plan;
-  plan.preferred_theta = par.preferred_theta;
   if (active) {
-    double pos[3];
-    valid_pose = load_pose<R2IK_POSE_MAT4>(M, i, true, pos, S.R);
-    if (valid_pose) {
-      Reach rc = is_reachable_R<false>(A, pos, S);
-      st = rc.state;
-      if (st == R2IK_STATE_REACHABLE) {
-        if (preferred_theta_works(A, S, rc.i0, rc.i1, par.preferred_theta)) {
-          theta = par.preferred_theta; found = true;
-        } else {
-          need_search = true;
-          double start, stop;
-          search_range(rc.i0, rc.i1, start, stop);
-          plan.L = make_linspace(start, stop, nb);
-          plan.T = make_elbow_test(A, S);
-        }
-      }
-    }
+    Reach rc;
+    valid_pose = disc_classify(A, par, M + 16 * i, S, rc, found, need_search);
+    st = rc.state;
+    if (found) theta = par.preferred_theta;
+    if (need_search) plan = disc_search_plan(A, par, S, rc);
   }
   unsigned pending = __ballot_sync(0xffffffffu, need_search);
   while (pending) {
@@ -532,38 +369,20 @@ k_ctl_discrete(const __grid_constant__ ArmConst A, const __grid_constant__ R2ikC
 #pragma unroll
   for (int k = 0; k < 7; ++k) { prev[k] = prev_joints[k]; cur[k] = current_joints[k]; }
   Solve S;
-  int st = R2IK_STATE_INVALID_ROTATION;
-  bool found = false;
-  double theta = 0.0, j[7], pos[3], i0 = 0.0, i1 = 0.0;
+  Reach rc;
+  bool found, need_search;
+  double theta = 0.0, j[7];
   int bits = 0;
-  const bool valid = load_pose<R2IK_POSE_MAT4>(M, i, true, pos, S.R);
-  if (valid) {
-    Reach rc = is_reachable_R<false>(A, pos, S);
-    st = rc.state; i0 = rc.i0; i1 = rc.i1;
-  }
   // The three sections below are kept apart by warp barriers: without them the compiler threads the preferred-theta
   // and the search paths separately through their own copies of the tail (get_joints + safety chain), and a warp runs
   // that tail twice at half the lanes (ncu: get_joints at 10 of 32 lanes for 64 % of the poses found).
-  bool need_search = false;
-  if (st == R2IK_STATE_REACHABLE) {
-    if (preferred_theta_works(A, S, i0, i1, par.preferred_theta)) { theta = par.preferred_theta; found = true; }
-    else need_search = true;
-  }
+  const bool valid = disc_classify(A, par, M + 16 * i, S, rc, found, need_search);
+  int st = rc.state;
+  if (found) theta = par.preferred_theta;
   __syncwarp(wmask);
   if (need_search) {
-    SearchPlan plan;
-    plan.preferred_theta = par.preferred_theta;
-    double start, stop;
-    search_range(i0, i1, start, stop);
-    plan.L = make_linspace(start, stop, par.nb_search_points);
-    plan.T = make_elbow_test(A, S);
-    double best;
-    int best_k;
-    if (!search_analytic(plan, par.nb_search_points, best, best_k))
-      search_strided(plan, par.nb_search_points, 0, 1, best, best_k);     // out-of-range magnitudes: scan
-    found = best < INFINITY;
-    if (found) theta = linspace_value(plan.L, best_k);
-    else st = R2IK_STATE_LIMITED_BY_SHOULDER;
+    found = disc_search(disc_search_plan(A, par, S, rc), par.nb_search_points, theta);
+    if (!found) st = R2IK_STATE_LIMITED_BY_SHOULDER;
   }
   __syncwarp(wmask);
   if (valid) {
@@ -788,15 +607,8 @@ k_reach_map(const __grid_constant__ ArmConst A, const __grid_constant__ f32::Arm
     __syncthreads();
     if (live) {
       for (int o = 0; o < m; ++o) {
-        bool esc;
-        int st = f32::reach_flag_mixed(A, AF, ps, px, sO[o], esc);
-        if (esc) {   // too close to call in FP32 (3e-4 of the pairs): the FP64 flag solve decides
-          const double *e = ori_euler + 3 * (size_t)(base + o);
-          Solve S;
-          S.p[0] = px; S.p[1] = py; S.p[2] = pz;
-          rot_from_euler_xyz(e[0], e[1], e[2], S.R);
-          st = solve_core<false, true>(A, S).state;
-        }
+        bool esc;   // too close to call in FP32: 3e-4 of the pairs
+        const int st = f32::reach_pair(A, AF, ps, px, py, pz, sO[o], ori_euler + 3 * (size_t)(base + o), esc);
         count += (st == R2IK_STATE_REACHABLE) ? 1u : 0u;
       }
     }
@@ -959,6 +771,19 @@ struct DeviceGuard {
 static inline bool misaligned16(const void *p) { return ((uintptr_t)p & 15) != 0; }
 static inline unsigned blocks_for(int64_t n) { return (unsigned)((n + R2IK_BLOCK - 1) / R2IK_BLOCK); }
 
+// Launch as a programmatic dependent of the preceding work on the stream: the kernel's blocks may be scheduled under its
+// predecessor's tail, and the kernel waits (griddepcontrol.wait) before it touches memory.
+template <typename... KArgs, typename... Args>
+static cudaError_t launch_pdl(void (*kernel)(KArgs...), unsigned grid, unsigned block, cudaStream_t s, Args... args) {
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(grid); cfg.blockDim = dim3(block); cfg.stream = s;
+  cfg.attrs = attr; cfg.numAttrs = 1;
+  return cudaLaunchKernelEx(&cfg, kernel, args...);
+}
+
 extern "C" {
 
 int r2ik_abi_version(void) { return R2IK_ABI_VERSION; }
@@ -1021,24 +846,15 @@ int r2ik_symik_solve_f64(r2ik_handle h, int pose_kind, const double *poses, cons
   DeviceGuard guard_(h->device);
   R2IK_CUDA(guard_.err, "cudaSetDevice");
   cudaStream_t s = (cudaStream_t)stream;
-  // staged (transposed, 128-bit) stores need 16-byte aligned output rows; anything else takes the scalar-store kernel
-  const bool staged = R2IK_K1_STAGED && (joints || elbow || interval) && !misaligned16(joints) && !misaligned16(elbow) && !misaligned16(interval);
-#define R2IK_LAUNCH_K1(KIND)                                                                                                          \
-  do {                                                                                                                                \
-    if (staged) k_symik_solve<KIND, true><<<blocks_for(n), R2IK_BLOCK, 0, s>>>(h->A, poses, theta, prev_joints, n, reachable, state, interval, joints, elbow); \
-    else if (R2IK_K1_PDL) {                                                                                                           \
-      cudaLaunchAttribute at_[1];                                                                                                     \
-      at_[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;                                                                 \
-      at_[0].val.programmaticStreamSerializationAllowed = 1;                                                                          \
-      cudaLaunchConfig_t cf_ = {};                                                                                                    \
-      cf_.gridDim = dim3(blocks_for(n)); cf_.blockDim = dim3(R2IK_BLOCK); cf_.stream = s; cf_.attrs = at_; cf_.numAttrs = 1;         \
-      R2IK_CUDA(cudaLaunchKernelEx(&cf_, k_symik_solve<KIND, false>, h->A, poses, theta, prev_joints, n, reachable, state, interval, joints, elbow), "k_symik_solve launch"); \
-    } else k_symik_solve<KIND, false><<<blocks_for(n), R2IK_BLOCK, 0, s>>>(h->A, poses, theta, prev_joints, n, reachable, state, interval, joints, elbow);       \
-  } while (0)
-  if (pose_kind == R2IK_POSE_MAT4) R2IK_LAUNCH_K1(R2IK_POSE_MAT4);
-  else if (pose_kind == R2IK_POSE_MAT34) R2IK_LAUNCH_K1(R2IK_POSE_MAT34);
-  else R2IK_LAUNCH_K1(R2IK_POSE_EULER6);
-#undef R2IK_LAUNCH_K1
+  const unsigned g = blocks_for(n);
+  cudaError_t e;
+  if (pose_kind == R2IK_POSE_MAT4)
+    e = launch_pdl(k_symik_solve<R2IK_POSE_MAT4>, g, R2IK_BLOCK, s, h->A, poses, theta, prev_joints, n, reachable, state, interval, joints, elbow);
+  else if (pose_kind == R2IK_POSE_MAT34)
+    e = launch_pdl(k_symik_solve<R2IK_POSE_MAT34>, g, R2IK_BLOCK, s, h->A, poses, theta, prev_joints, n, reachable, state, interval, joints, elbow);
+  else
+    e = launch_pdl(k_symik_solve<R2IK_POSE_EULER6>, g, R2IK_BLOCK, s, h->A, poses, theta, prev_joints, n, reachable, state, interval, joints, elbow);
+  R2IK_CUDA(e, "k_symik_solve launch");
   R2IK_CUDA(cudaGetLastError(), "k_symik_solve launch");
   return 0;
 }
@@ -1071,28 +887,19 @@ int r2ik_symik_solve_f32(r2ik_handle h, int pose_kind, const float *poses, const
   const unsigned eb = (unsigned)(ew < 2368 ? ew : 2368);
   // count reset, first pass and second pass are a chain of programmatic dependents: each is scheduled under its
   // predecessor's tail and waits (griddepcontrol.wait) before it touches memory
-  cudaLaunchAttribute eattr[1];
-  eattr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  eattr[0].val.programmaticStreamSerializationAllowed = 1;
-  cudaLaunchConfig_t ecfg = {};
-  ecfg.gridDim = dim3(1); ecfg.blockDim = dim3(32); ecfg.dynamicSmemBytes = 0; ecfg.stream = s;
-  ecfg.attrs = eattr; ecfg.numAttrs = 1;
-  R2IK_CUDA(cudaLaunchKernelEx(&ecfg, k_zero_u32, n_escalated), "k_zero_u32 launch");
-  const uint32_t *esc_c = escalated_idx;
-  const unsigned *nesc_c = n_escalated;
-  ecfg.blockDim = dim3(R2IK_BLOCK);
-#define R2IK_LAUNCH_K1F(KIND)                                                                                                       \
-  do {                                                                                                                              \
-    ecfg.gridDim = dim3(blocks_for(n));                                                                                             \
-    R2IK_CUDA(cudaLaunchKernelEx(&ecfg, k_symik_solve_f32<KIND>, h->A, h->AF, poses, theta, n, reachable, state, interval, joints,  \
-                                 elbow, escalated_idx, n_escalated), "k_symik_solve_f32 launch");                                    \
-    ecfg.gridDim = dim3(eb); ecfg.blockDim = dim3(32);                                                                              \
-    R2IK_CUDA(cudaLaunchKernelEx(&ecfg, k_symik_escalated_f32<KIND>, h->A, poses, theta, prev_joints, reachable, state, interval,   \
-                                 joints, elbow, esc_c, nesc_c), "k_symik_escalated_f32 launch");                                     \
-  } while (0)
-  if (pose_kind == R2IK_POSE_MAT4) R2IK_LAUNCH_K1F(R2IK_POSE_MAT4);
-  else R2IK_LAUNCH_K1F(R2IK_POSE_EULER6);
-#undef R2IK_LAUNCH_K1F
+  R2IK_CUDA(launch_pdl(k_zero_u32, 1, 32, s, n_escalated), "k_zero_u32 launch");
+  const bool mat4 = pose_kind == R2IK_POSE_MAT4;
+  const unsigned g = blocks_for(n);
+  R2IK_CUDA(mat4 ? launch_pdl(k_symik_solve_f32<R2IK_POSE_MAT4>, g, R2IK_BLOCK, s, h->A, h->AF, poses, theta, n, reachable, state,
+                              interval, joints, elbow, escalated_idx, n_escalated)
+                 : launch_pdl(k_symik_solve_f32<R2IK_POSE_EULER6>, g, R2IK_BLOCK, s, h->A, h->AF, poses, theta, n, reachable, state,
+                              interval, joints, elbow, escalated_idx, n_escalated),
+            "k_symik_solve_f32 launch");
+  R2IK_CUDA(mat4 ? launch_pdl(k_symik_escalated_f32<R2IK_POSE_MAT4>, eb, 32, s, h->A, poses, theta, prev_joints, reachable, state,
+                              interval, joints, elbow, escalated_idx, n_escalated)
+                 : launch_pdl(k_symik_escalated_f32<R2IK_POSE_EULER6>, eb, 32, s, h->A, poses, theta, prev_joints, reachable, state,
+                              interval, joints, elbow, escalated_idx, n_escalated),
+            "k_symik_escalated_f32 launch");
   R2IK_CUDA(cudaGetLastError(), "k_symik_solve_f32 launch");
   return 0;
 }
@@ -1203,9 +1010,6 @@ int r2ik_ctl_discrete_scan_f64(r2ik_handle h, const R2ikCtlParams *par, const do
   return ctl_discrete_launch(true, h, par, M, n, prev_joints, current_joints, joints, reachable, state, emergency, stream);
 }
 
-#ifndef R2IK_K2C_PDL
-#define R2IK_K2C_PDL 1
-#endif
 int64_t r2ik_ctl_discrete_workspace_bytes(int64_t n) { return n < 0 ? -1 : (int64_t)disc_ws_bytes(n); }
 
 int r2ik_ctl_discrete_compact_f64(r2ik_handle h, const R2ikCtlParams *par, const double *M, int64_t n, const double *prev_joints,
@@ -1229,22 +1033,12 @@ int r2ik_ctl_discrete_compact_f64(r2ik_handle h, const R2ikCtlParams *par, const
   // consts is an ordinary launch (it waits for everything before it on the stream); the three passes are programmatic
   // dependents of their predecessors (r2ik_discrete_compact.cuh)
   k_disc_consts<<<1, 32, 0, s>>>(*par, prev_joints, current_joints, w.hdr);
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = R2IK_K2C_PDL;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(lb); cfg.blockDim = dim3(R2IK_BLOCK); cfg.dynamicSmemBytes = 0; cfg.stream = s;
-  cfg.attrs = attr; cfg.numAttrs = 1;
-  const double *Mc = M, *prevc = prev_joints;
-  const double *planc = w.plan, *thetac = w.finish_theta;
-  const uint32_t *sidxc = w.search_idx, *fidxc = w.finish_idx;
-  const DiscHeader *hdrc = w.hdr;
-  R2IK_CUDA(cudaLaunchKernelEx(&cfg, k_disc_classify, h->A, *par, Mc, n, w.hdr, w.plan, w.finish_theta, w.search_idx, w.finish_idx,
-                               joints, reachable, state, emergency), "k_disc_classify launch");
-  R2IK_CUDA(cudaLaunchKernelEx(&cfg, k_disc_search, *par, w.hdr, planc, w.finish_theta, sidxc, w.finish_idx, joints, reachable, state,
-                               emergency), "k_disc_search launch");
-  R2IK_CUDA(cudaLaunchKernelEx(&cfg, k_disc_finish, h->A, *par, Mc, prevc, hdrc, thetac, fidxc, joints, reachable, state, emergency),
-            "k_disc_finish launch");
+  R2IK_CUDA(launch_pdl(k_disc_classify, lb, R2IK_BLOCK, s, h->A, *par, M, n, w.hdr, w.plan, w.finish_theta, w.search_idx,
+                       w.finish_idx, joints, reachable, state, emergency), "k_disc_classify launch");
+  R2IK_CUDA(launch_pdl(k_disc_search, lb, R2IK_BLOCK, s, *par, w.hdr, w.plan, w.finish_theta, w.search_idx, w.finish_idx, joints,
+                       reachable, state, emergency), "k_disc_search launch");
+  R2IK_CUDA(launch_pdl(k_disc_finish, lb, R2IK_BLOCK, s, h->A, *par, M, prev_joints, w.hdr, w.finish_theta, w.finish_idx, joints,
+                       reachable, state, emergency), "k_disc_finish launch");
   R2IK_CUDA(cudaGetLastError(), "k_disc_* launch");
   return 0;
 }

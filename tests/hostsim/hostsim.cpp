@@ -1,28 +1,26 @@
-// TEST-ONLY host harness: compiles the device solver source (r2ik_device.cuh /
-// r2ik_control.cuh, all __host__ __device__) with g++ and loops over poses on the CPU, so the
-// kernel *logic* is checked against the golden fixtures in the GPU-less CI.  It is not part
-// of libr2ik.so, is never imported by the package, and is no fallback for anything.
+// TEST-ONLY host harness: compiles the device solver source (the csrc headers, all __host__ __device__) with g++ and
+// loops over poses / waypoints / pairs on the CPU, calling the same per-item functions the kernels call, so the kernel
+// *logic* is checked against the golden fixtures in the GPU-less CI.  It is not part of libr2ik.so, is never imported
+// by the package, and is no fallback for anything.
 #include <cstring>
 #include <vector>
 #include <cstdint>
+#include <type_traits>
 
 #include "../../reachy2_symbolic_ik_b200/csrc/r2ik_control.cuh"
 #include "../../reachy2_symbolic_ik_b200/csrc/r2ik_cont_codes.cuh"
+#include "../../reachy2_symbolic_ik_b200/csrc/r2ik_discrete_compact.cuh"
 #define R2IK_F32_DEBUG 1
 #include "../../reachy2_symbolic_ik_b200/csrc/r2ik_device_f32.cuh"
 #include "../../reachy2_symbolic_ik_b200/csrc/r2ik_host.h"
 
 using namespace r2ik;
 
-// mirrors load_pose<KIND> of r2ik_kernels.cu
-static bool load_pose(int kind, const double *p, bool snap, double pos[3], double R[9]) {
-  if (kind == R2IK_POSE_EULER6) {
-    for (int k = 0; k < 3; ++k) pos[k] = p[k];
-    rot_from_euler_xyz(p[3], p[4], p[5], R);
-    return true;
-  }
-  pos[0] = p[3]; pos[1] = p[7]; pos[2] = p[11];
-  return rotation_from_mat4(p, snap, R);
+// f(std::integral_constant<int, KIND>) for the pose layout `kind` (EULER6, anything else MAT4)
+template <typename F>
+static void by_kind(int kind, F f) {
+  if (kind == R2IK_POSE_EULER6) f(std::integral_constant<int, R2IK_POSE_EULER6>());
+  else f(std::integral_constant<int, R2IK_POSE_MAT4>());
 }
 
 extern "C" {
@@ -67,37 +65,26 @@ void hs_symik_batch(const R2ikArmConfig *cfg, int kind, const double *poses, con
                     uint8_t *reach, uint8_t *state, double *interval, double *joints, double *elbow) {
   ArmConst A; R2ikArmConstants pub;
   derive_constants(*cfg, A, pub);
-  int stride = kind == R2IK_POSE_EULER6 ? 6 : 16;
-  for (int64_t i = 0; i < n; ++i) {
-    double pos[3];
-    Solve S;
-    for (int k = 0; k < 7; ++k) joints[7 * i + k] = NAN;
-    for (int k = 0; k < 3; ++k) elbow[3 * i + k] = NAN;
-    interval[2 * i] = NAN; interval[2 * i + 1] = NAN;
-    if (!load_pose(kind, poses + i * stride, false, pos, S.R)) { reach[i] = 0; state[i] = R2IK_STATE_INVALID_ROTATION; continue; }
-    Reach rc = is_reachable_R<false>(A, pos, S);
-    state[i] = (uint8_t)rc.state;
-    reach[i] = rc.state == R2IK_STATE_REACHABLE;
-    if (reach[i]) {
+  by_kind(kind, [&](auto K) {
+    for (int64_t i = 0; i < n; ++i) {
+      Solve S;
+      const Reach rc = symik_reach<K()>(A, poses + pose_stride(K()) * i, S);
+      reach[i] = rc.state == R2IK_STATE_REACHABLE;
+      state[i] = (uint8_t)rc.state;
       interval[2 * i] = rc.i0; interval[2 * i + 1] = rc.i1;
-      if (theta) get_joints(A, S, theta[i], 0.0, 0.0, joints + 7 * i, elbow + 3 * i);
-      else get_joints_cs(A, S, rc.c0, rc.s0, 0.0, 0.0, joints + 7 * i, elbow + 3 * i);
+      symik_joints(A, S, rc, theta ? theta + i : nullptr, 0.0, 0.0, joints + 7 * i, elbow + 3 * i);
     }
-  }
+  });
 }
 
 void hs_no_limits_batch(const R2ikArmConfig *cfg, int kind, const double *poses, const double *theta, int64_t n,
                         double *joints, double *elbow) {
   ArmConst A; R2ikArmConstants pub;
   derive_constants(*cfg, A, pub);
-  int stride = kind == R2IK_POSE_EULER6 ? 6 : 16;
-  for (int64_t i = 0; i < n; ++i) {
-    double pos[3];
-    Solve S;
-    load_pose(kind, poses + i * stride, false, pos, S.R);
-    is_reachable_R<true>(A, pos, S);
-    get_joints(A, S, theta[i], 0.0, 0.0, joints + 7 * i, elbow + 3 * i);
-  }
+  by_kind(kind, [&](auto K) {
+    for (int64_t i = 0; i < n; ++i)
+      symik_no_limits<K()>(A, poses + pose_stride(K()) * i, theta + i, nullptr, joints + 7 * i, elbow + 3 * i);
+  });
 }
 
 void hs_ctl_discrete_batch(const R2ikArmConfig *cfg, const R2ikCtlParams *par, const double *M, int64_t n,
@@ -106,119 +93,66 @@ void hs_ctl_discrete_batch(const R2ikArmConfig *cfg, const R2ikCtlParams *par, c
   ArmConst A; R2ikArmConstants pub;
   derive_constants(*cfg, A, pub);
   for (int64_t i = 0; i < n; ++i) {
-    double pos[3];
     Solve S;
-    if (!load_pose(R2IK_POSE_MAT4, M + 16 * i, true, pos, S.R)) {
-      for (int k = 0; k < 7; ++k) joints[7 * i + k] = NAN;
-      reach[i] = 0; state[i] = R2IK_STATE_INVALID_ROTATION; emg[i] = 0;
-      continue;
-    }
-    Reach rc = is_reachable_R<false>(A, pos, S);
-    int st = rc.state;
-    bool ok = st == R2IK_STATE_REACHABLE;
+    Reach rc;
+    bool found, need_search;
     double theta = 0.0;
-    if (ok) {
-      // mirrors k_ctl_discrete: preferred-theta shortcut, else the analytic arg-min over the K samples (scan fallback)
-      if (preferred_theta_works(A, S, rc.i0, rc.i1, par->preferred_theta)) {
-        theta = par->preferred_theta;
-      } else {
-        SearchPlan plan;
-        plan.preferred_theta = par->preferred_theta;
-        double start, stop;
-        search_range(rc.i0, rc.i1, start, stop);
-        plan.L = make_linspace(start, stop, par->nb_search_points);
-        plan.T = make_elbow_test(A, S);
-        double best;
-        int best_k;
-        if (!search_analytic(plan, par->nb_search_points, best, best_k))
-          search_strided(plan, par->nb_search_points, 0, 1, best, best_k);
-        ok = best < INFINITY;
-        if (ok) theta = linspace_value(plan.L, best_k);
-        else st = R2IK_STATE_LIMITED_BY_SHOULDER;
-      }
+    const bool valid = disc_classify(A, *par, M + 16 * i, S, rc, found, need_search);
+    int st = rc.state;
+    if (found) theta = par->preferred_theta;
+    if (need_search) {
+      found = disc_search(disc_search_plan(A, *par, S, rc), par->nb_search_points, theta);
+      if (!found) st = R2IK_STATE_LIMITED_BY_SHOULDER;
     }
-    emg[i] = (uint8_t)discrete_finish(A, *par, S, ok, theta, prev, cur, joints + 7 * i);
-    reach[i] = ok; state[i] = (uint8_t)st;
+    if (valid) emg[i] = (uint8_t)discrete_finish(A, *par, S, found, theta, prev, cur, joints + 7 * i);
+    else {
+      for (int k = 0; k < 7; ++k) joints[7 * i + k] = NAN;
+      emg[i] = 0;
+    }
+    reach[i] = found; state[i] = (uint8_t)st;
   }
 }
 
-// (the CUDA header r2ik_discrete_compact.cuh is device-only; its two host-visible definitions are mirrored here)
-struct DiscHeader { unsigned n_search, n_finish; int nf_bits; double nf_joints[7]; };
-constexpr uint32_t kDiscLiteral = 0x80000000u;
-
-// Host twin of r2ik_ctl_discrete_compact_f64 (csrc/r2ik_discrete_compact.cuh): the three passes run one after the other
-// over the same lists -- entries with the literal-solve flag in bit 31, the 64-byte search plan, the finish pass redoing
-// only the elbow circle -- with the appends in `order` (0: ascending, 1: descending pose index) to show that the result
-// does not depend on the order the blocks arrive in.  n_lists[0..2] receive the list lengths and the number of finish
-// entries that carry the literal-solve flag.
+// The three passes of r2ik_ctl_discrete_compact_f64 one after the other over the same lists, with the appends in `order`
+// (0: ascending, 1: descending pose index) to show that the result does not depend on the order the blocks arrive in.
+// n_lists[0..2] receive the list lengths and the number of finish entries that carry the literal-solve flag.
 void hs_ctl_discrete_compact_batch(const R2ikArmConfig *cfg, const R2ikCtlParams *par, const double *M, int64_t n,
                                    const double *prev, const double *cur, int order, double *joints, uint8_t *reach,
                                    uint8_t *state, uint8_t *emg, int64_t *n_lists) {
   ArmConst A; R2ikArmConstants pub;
   derive_constants(*cfg, A, pub);
   DiscHeader hdr;
-  {   // k_disc_consts
-    double j[7];
-    for (int k = 0; k < 7; ++k) j[k] = cur[k];
-    hdr.nf_bits = safety_checks(j, prev, par->orbita3d_max_angle);
-    for (int k = 0; k < 7; ++k) hdr.nf_joints[k] = j[k];
-    hdr.n_search = 0; hdr.n_finish = 0;
-  }
+  disc_header_init(&hdr, *par, prev, cur);
   std::vector<uint32_t> search_idx((size_t)n), finish_idx((size_t)n);
   std::vector<double> plan(8 * (size_t)n), finish_theta((size_t)n);
-  auto store_final = [&](int64_t i, int st) {
-    const bool invalid = st == R2IK_STATE_INVALID_ROTATION;
-    for (int k = 0; k < 7; ++k) joints[7 * i + k] = invalid ? NAN : hdr.nf_joints[k];
-    reach[i] = 0; state[i] = (uint8_t)st; emg[i] = invalid ? 0 : (uint8_t)hdr.nf_bits;
-  };
   for (int64_t q = 0; q < n; ++q) {   // k_disc_classify
     const int64_t i = order ? n - 1 - q : q;
-    double pos[3];
     Solve S;
-    int st = R2IK_STATE_INVALID_ROTATION;
-    bool shortcut = false, need_search = false;
-    double i0 = 0.0, i1 = 0.0;
+    Reach rc;
+    bool shortcut, need_search;
     uint32_t tag = (uint32_t)i;
-    if (load_pose(R2IK_POSE_MAT4, M + 16 * i, true, pos, S.R)) {
-      Reach rc = is_reachable_R<false>(A, pos, S);
-      st = rc.state; i0 = rc.i0; i1 = rc.i1;
-      if (rc.literal) tag |= kDiscLiteral;
-      if (st == R2IK_STATE_REACHABLE) {
-        shortcut = preferred_theta_works(A, S, i0, i1, par->preferred_theta);
-        need_search = !shortcut;
-      }
-    }
+    disc_classify(A, *par, M + 16 * i, S, rc, shortcut, need_search);
+    if (rc.literal) tag |= kDiscLiteral;
     if (need_search) {
-      const ElbowTest T = make_elbow_test(A, S);
       const size_t k = hdr.n_search++;
       search_idx[k] = tag;
-      double *p = &plan[8 * k];
-      p[0] = i0; p[1] = i1; p[2] = T.A1; p[3] = T.B1; p[4] = T.C1; p[5] = T.A2; p[6] = T.B2; p[7] = T.C2;
+      disc_plan_pack(&plan[8 * k], A, S, rc.i0, rc.i1);
     } else if (shortcut) {
       const size_t k = hdr.n_finish++;
       finish_idx[k] = tag; finish_theta[k] = par->preferred_theta;
     } else {
-      store_final(i, st);
+      disc_store_final(&hdr, i, rc.state, joints, reach, state, emg);
     }
   }
   n_lists[0] = hdr.n_search;
   for (size_t k = 0; k < hdr.n_search; ++k) {   // k_disc_search
     const uint32_t tag = search_idx[k];
-    const double *p = &plan[8 * k];
-    SearchPlan P;
-    P.preferred_theta = par->preferred_theta;
-    double start, stop;
-    search_range(p[0], p[1], start, stop);
-    P.L = make_linspace(start, stop, par->nb_search_points);
-    P.T.A1 = p[2]; P.T.B1 = p[3]; P.T.C1 = p[4]; P.T.A2 = p[5]; P.T.B2 = p[6]; P.T.C2 = p[7];
-    double best;
-    int best_k;
-    if (!search_analytic(P, par->nb_search_points, best, best_k)) search_strided(P, par->nb_search_points, 0, 1, best, best_k);
-    if (best < INFINITY) {
+    double theta;
+    if (disc_search(disc_plan_unpack(*par, &plan[8 * k]), par->nb_search_points, theta)) {
       const size_t f = hdr.n_finish++;
-      finish_idx[f] = tag; finish_theta[f] = linspace_value(P.L, best_k);
+      finish_idx[f] = tag; finish_theta[f] = theta;
     } else {
-      store_final((int64_t)(tag & ~kDiscLiteral), R2IK_STATE_LIMITED_BY_SHOULDER);
+      disc_store_final(&hdr, (int64_t)(tag & ~kDiscLiteral), R2IK_STATE_LIMITED_BY_SHOULDER, joints, reach, state, emg);
     }
   }
   n_lists[1] = hdr.n_finish;
@@ -227,12 +161,7 @@ void hs_ctl_discrete_compact_batch(const R2ikArmConfig *cfg, const R2ikCtlParams
     const uint32_t tag = finish_idx[k];
     n_lists[2] += (tag & kDiscLiteral) != 0;
     const int64_t i = tag & ~kDiscLiteral;
-    Solve S;
-    double pos[3];
-    load_pose(R2IK_POSE_MAT4, M + 16 * i, true, pos, S.R);
-    if (tag & kDiscLiteral) is_reachable_R<false>(A, pos, S);
-    else circle_of_reachable(A, pos, S);
-    emg[i] = (uint8_t)discrete_finish(A, *par, S, true, finish_theta[k], prev, prev, joints + 7 * i);
+    emg[i] = (uint8_t)disc_finish_listed(A, *par, M + 16 * i, (tag & kDiscLiteral) != 0, finish_theta[k], prev, joints + 7 * i);
     reach[i] = 1; state[i] = R2IK_STATE_REACHABLE;
   }
 }
@@ -285,17 +214,7 @@ void hs_ctl_continuous_phased_batch(const R2ikArmConfig *cfg, const R2ikCtlParam
       double j[7];
       bool serial = false;
       for (int q = 0; q < 7; ++q) j[q] = NAN;
-      if (c != R2IK_WP_INVALID) {
-        const double *m = M + 16 * k;
-        Solve S; double pos[3] = {m[3], m[7], m[11]};
-        rotation_from_mat4(m, true, S.R);
-        if (c == R2IK_WP_UNREACHABLE) is_reachable_R<true>(A, pos, S); else circle_of_reachable(A, pos, S);
-        double sn, cs_, E[3];
-        sincos_any(ws[k], sn, cs_);
-        serial = !get_joints_impl<false>(A, S, cs_, sn, 0.0, 0.0, j, E);
-        if (force_serial_mod > 0 && k % force_serial_mod == 0) serial = true;
-        if (!serial) limit_orbita3d_wrist(j, par->orbita3d_max_angle);
-      }
+      if (c != R2IK_WP_INVALID) serial = cont_raw_joints_item(A, *par, M + 16 * k, c, ws + k, k, force_serial_mod, j);
       const bool ordinary = c != R2IK_WP_INVALID && !serial;
       unsigned cd = (ordinary && w > 0 && prev_ordinary) ? cont_wind_code(j, jp) : cont_irregular_code(serial ? (c | R2IK_WP_SERIAL) : c);
       codes[k] = (uint16_t)cd;
@@ -305,59 +224,38 @@ void hs_ctl_continuous_phased_batch(const R2ikArmConfig *cfg, const R2ikCtlParam
     }
   }
   for (int64_t t = 0; t < T; ++t) {                          // k_cont_finish_codes
-    const size_t base = (size_t)t * W;
+    const double *Mt = M + 16 * (size_t)t * W;
     auto serial = [&](int w, int kind, double theta, double p0, double p2, double *out) {
-      const double *m = M + 16 * (base + w);
-      Solve S; double pos[3] = {m[3], m[7], m[11]};
-      rotation_from_mat4(m, true, S.R);
-      if (kind != R2IK_WP_UNREACHABLE) is_reachable_R<false>(A, pos, S);
-      cont_raw_joints(A, *par, kind, pos, S, theta, p0, p2, out);
+      cont_serial_joints(A, *par, Mt + 16 * (size_t)w, kind, theta, p0, p2, out);
     };
+    const size_t base = (size_t)t * W;
     cont_finish_codes_trajectory(W, cur_joints + 7 * t, st[t], ws + base, codes + base, joints + 7 * base, reach + base, state + base, serial);
   }
 }
 
-// K1-f32 (r2ik_device_f32.cuh): the FP32 fast solve with FP64 escalation, mirroring k_symik_solve_f32.
-// mode: 0 = as the kernel (escalate flagged poses), 1 = never escalate (raw FP32 results, to measure them).
-// k_ctl_ctor_theta of r2ik_kernels.cu (ControlIK.__init__'s previous_theta seed, ctl:142-159)
 double hs_ctl_ctor_theta(const R2ikArmConfig *cfg, double preferred_theta, const double *rows, int n_rows, const double *current_pose) {
   ArmConst A; R2ikArmConstants pub;
   derive_constants(*cfg, A, pub);
-  Solve S;
-  const double cpos[3] = {current_pose[3], current_pose[7], current_pose[11]};
-  if (!rotation_from_mat4(current_pose, true, S.R) || is_reachable_R<true>(A, cpos, S).state != R2IK_STATE_REACHABLE) return NAN;
-  return ctor_previous_theta(A, S, rows, n_rows, preferred_theta);
+  return ctl_ctor_theta(A, current_pose, rows, n_rows, preferred_theta);
 }
 
-// get_elbow_position(thetas[i][k]) + the projection predicate, as k_elbow_positions<KIND, NO_LIMITS> of r2ik_kernels.cu
 void hs_elbow_positions(const R2ikArmConfig *cfg, int kind, const double *poses, const double *thetas, int K, int64_t n,
                         int no_limits, double *elbows, uint8_t *projected) {
   ArmConst A; R2ikArmConstants pub;
   derive_constants(*cfg, A, pub);
-  int stride = kind == R2IK_POSE_EULER6 ? 6 : 16;
-  for (int64_t i = 0; i < n; ++i) {
-    double pos[3];
-    Solve S;
-    bool ok = load_pose(kind, poses + i * stride, false, pos, S.R);
-    if (ok) {
-      const int st = no_limits ? is_reachable_R<true>(A, pos, S).state : is_reachable_R<false>(A, pos, S).state;
-      ok = st == R2IK_STATE_REACHABLE || (!no_limits && st == R2IK_STATE_LIMITED_BY_WRIST);
+  by_kind(kind, [&](auto KI) {
+    for (int64_t i = 0; i < n; ++i) {
+      const double *row = poses + pose_stride(KI()) * i;
+      Solve S;
+      const bool circle = no_limits ? pose_elbow_circle<KI(), true>(A, row, S) : pose_elbow_circle<KI(), false>(A, row, S);
+      for (int k = 0; k < K; ++k)
+        projected[i * K + k] = elbow_on_circle(A, S, circle, thetas + (i * K + k), elbows + (i * K + k) * 3);
     }
-    for (int k = 0; k < K; ++k) {
-      double E[3] = {NAN, NAN, NAN};
-      bool proj = false;
-      if (ok) {
-        double st, ct;
-        sincos_any(thetas[i * K + k], st, ct);
-        elbow_position_cs(S, ct, st, E);
-        proj = E[2] > (E[0] - A.es[0]) * A.sing_coeff + A.es[2] - A.sing_offset;
-      }
-      for (int c = 0; c < 3; ++c) elbows[(i * K + k) * 3 + c] = E[c];
-      projected[i * K + k] = proj;
-    }
-  }
+  });
 }
 
+// K1-f32 (r2ik_device_f32.cuh): the FP32 fast solve with FP64 escalation, as k_symik_solve_f32 + k_symik_escalated_f32.
+// mode: 0 = as the kernels (escalate flagged poses), 1 = never escalate (raw FP32 results, to measure them).
 void hs_symik_batch_f32(const R2ikArmConfig *cfg, int kind, const float *poses, const float *theta, int64_t n, int mode,
                         uint8_t *reach, uint8_t *state, float *interval, float *joints, float *elbow, uint8_t *escalated) {
   ArmConst A; R2ikArmConstants pub;
@@ -407,7 +305,7 @@ void hs_search_compare(const double *plans, int64_t n, int nb, double *best_scan
   }
 }
 
-// K4 with the mixed-precision flag (reach_flag_mixed) and FP64 escalation, mirroring k_reach_map.
+// K4 with the mixed-precision flag and FP64 escalation (reach_pair, as k_reach_map).
 // mode 0: as the kernel; mode 1: never escalate (to measure what the bands catch).  n_esc: escalated pairs.
 void hs_reach_map_mixed(const R2ikArmConfig *cfg, const double *origin, const double *step, const int32_t *dims,
                         const double *ori_euler, int32_t ori_begin, int32_t ori_end, int mode, uint32_t *counts,
@@ -417,12 +315,12 @@ void hs_reach_map_mixed(const R2ikArmConfig *cfg, const double *origin, const do
   f32::ArmConstF F;
   f32::narrow_constants(A, F);
   const int no = ori_end - ori_begin;
-  f32::OriConst *O = new f32::OriConst[no];
-  double *Rs = new double[9 * (size_t)no];
+  std::vector<f32::OriConst> O((size_t)no);
   for (int o = 0; o < no; ++o) {
     const double *e = ori_euler + 3 * (size_t)(ori_begin + o);
-    rot_from_euler_xyz(e[0], e[1], e[2], Rs + 9 * o);
-    O[o] = f32::make_ori_const(A, Rs + 9 * o);
+    double R[9];
+    rot_from_euler_xyz(e[0], e[1], e[2], R);
+    O[o] = f32::make_ori_const(A, R);
   }
   *n_esc = 0; *n_live_pairs = 0;
   for (int ix = 0; ix < dims[0]; ++ix)
@@ -434,21 +332,15 @@ void hs_reach_map_mixed(const R2ikArmConfig *cfg, const double *origin, const do
           const double ps[3] = {px - A.s[0], py - A.s[1], pz - A.s[2]};
           for (int o = 0; o < no; ++o) {
             bool esc = false;
-            int st = f32::reach_flag_mixed(A, F, ps, px, O[o], esc);
+            const int st = mode == 1 ? f32::reach_flag_mixed(A, F, ps, px, O[o], esc)
+                                     : f32::reach_pair(A, F, ps, px, py, pz, O[o], ori_euler + 3 * (size_t)(ori_begin + o), esc);
             ++*n_live_pairs;
             if (esc) ++*n_esc;
-            if (esc && mode == 0) {
-              Solve S;
-              S.p[0] = px; S.p[1] = py; S.p[2] = pz;
-              for (int k = 0; k < 9; ++k) S.R[k] = Rs[9 * o + k];
-              st = solve_core<false, true>(A, S).state;
-            }
             count += st == R2IK_STATE_REACHABLE;
           }
         }
         counts[((size_t)ix * dims[1] + iy) * dims[2] + iz] = count;
       }
-  delete[] O; delete[] Rs;
 }
 
 }  // extern "C"
