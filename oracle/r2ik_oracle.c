@@ -191,6 +191,16 @@ static int quat_from_matrix(const double min[3][3], double q[4]) {
       if (!(fabs(g - e) <= 1e-12 + 1e-5 * fabs(e))) orthogonal = 0;
     }
   if (!orthogonal) {
+    /* U @ Vt does not depend on the scale of the block, while the iteration only halves a scale error per step:
+     * a block whose largest entry lies outside [2^-4, 2^4] is first scaled to unit size by an exact power of two. */
+    double mx = 0.0;
+    for (int i = 0; i < 3; i++)
+      for (int j = 0; j < 3; j++) mx = fmax(mx, fabs(m[i][j]));
+    if (mx < 0.0625 || (mx > 16.0 && mx < INFINITY)) {
+      int e = ilogb(mx);
+      for (int i = 0; i < 3; i++)
+        for (int j = 0; j < 3; j++) m[i][j] = ldexp(m[i][j], -e);
+    }
     for (int it = 0; it < 60; it++) {
       double y[3][3], delta = 0.0;
       inv3_transpose(m, y);

@@ -126,22 +126,26 @@ R2IK_HD double pymod(double a, double m) {
 }
 
 // pymod(x, 2 pi) for the arguments the controller produces.  Python's float % is fmod (exact) plus at
-// most one rounded `+ m`.  For -2 pi <= x < 8 pi the exact remainder is reached by subtracting 4 pi /
+// most one rounded `+ m`.  For 0 <= x < 8 pi the exact remainder is reached by subtracting 4 pi /
 // 2 pi when x is at least that: 2 pi and 4 pi are exact multiples of the same double and every
 // difference below is exactly representable (both operands are multiples of the ulp of the result
 // range), so each step is error-free and the value is bit-identical to fmod's.  Negative x in
-// [-2 pi, 0) is Python's `fmod(x) + m`, one rounded add, as here.  Anything else takes pymod().
-R2IK_HD double pymod_2pi(double x) {
+// [-2 pi, 0) is Python's `fmod(x) + m`, one rounded add and nothing more: for -x below half an ulp of
+// 2 pi that sum rounds to 2 pi itself, which Python returns as it is.  Anything else takes pymod().
+// For x = -0 this returns -0 where Python gives +0: pymod_2pi below adds the fix, angle_diff (whose
+// argument is never -0) does without it.
+R2IK_HD double pymod_2pi_not_minus_zero(double x) {
   const double two_pi = R2IK_WRAP(1), four_pi = R2IK_WRAP(2);
   if (!(x >= -two_pi && x < R2IK_WRAP(3))) return pymod(x, kTwoPi);
-  double r = x < 0.0 ? x + two_pi : x;
-  r = r >= four_pi ? r - four_pi : r;
+  double r = x >= four_pi ? x - four_pi : x;
   r = r >= two_pi ? r - two_pi : r;
-  return r;
+  return x < 0.0 ? x + two_pi : r;
 }
+// A zero remainder is +0: `+ 0.0` turns -0 into +0 and leaves every other value as it is.
+R2IK_HD double pymod_2pi(double x) { return pymod_2pi_not_minus_zero(x) + 0.0; }
 
-// utl:486-490
-R2IK_HD double angle_diff(double a, double b) { return pymod_2pi((a - b) + R2IK_WRAP(0)) - R2IK_WRAP(0); }
+// utl:486-490.  (a - b) + pi is never -0 (a sum is -0 only when both terms are).
+R2IK_HD double angle_diff(double a, double b) { return pymod_2pi_not_minus_zero((a - b) + R2IK_WRAP(0)) - R2IK_WRAP(0); }
 
 // np.isclose(a, b), rtol 1e-5, atol 1e-8 (asymmetric in b)
 R2IK_HD bool np_isclose(double a, double b) { return fabs(a - b) <= 1e-8 + 1e-5 * fabs(b); }
@@ -259,7 +263,16 @@ R2IK_HD double det3(const double m[9]) {
 // two iterates agree to 1e-8 the next one is the fixed point to rounding, so one more step is taken and
 // the loop ends (waiting for the step itself to fall below one ulp, as an earlier version did, never
 // happens when the last bits keep flipping -- 60 iterations for every nearly-orthonormal input).
+// The plain iteration only halves a scale error per step (a block scaled by 10^k needs ~3.3 |k| steps, far more than
+// the 60 allowed), so a block whose largest entry lies outside [2^-4, 2^4] is first brought to unit size by an exact
+// power-of-two scaling -- the polar factor does not depend on the scale.  Ordinary blocks are iterated as they are.
 R2IK_HD void polar_orthogonalize(double m[9]) {
+  double mx = 0.0;
+  for (int k = 0; k < 9; ++k) mx = fmax(mx, fabs(m[k]));
+  if (mx < 0.0625 || (mx > 16.0 && mx < INFINITY)) {
+    const int e = ilogb(mx);
+    for (int k = 0; k < 9; ++k) m[k] = ldexp(m[k], -e);
+  }
   bool last = false;
   for (int it = 0; it < 60; ++it) {
     double id = 1.0 / det3(m);
@@ -522,8 +535,9 @@ R2IK_HD int reach_prechecks(const ArmConst &A, double &px, double &py, double &p
   bool outside = dg2 > L2;
   if (fabs(dg2 - L2) <= 1e-12) outside = sqrt(dg2) > A.max_arm_length;
   if (outside) {
-    double dg = sqrt_nonneg(dg2);
-    double sc = div_fast(A.max_arm_length, dg + A.proj_margin);
+    // a goal beyond ~1.3e154 m overflows dg2: the reference's norm is then inf and the goal lands on the shoulder
+    // (dx / inf = 0), where sqrt_nonneg(inf) would be NaN
+    double sc = dg2 < INFINITY ? div_fast(A.max_arm_length, sqrt_nonneg(dg2) + A.proj_margin) : 0.0;
     px = A.s[0] + dx * sc;
     py = A.s[1] + dy * sc;
     pz = A.s[2] + dz * sc;

@@ -50,6 +50,46 @@ def hs_symik(hs, cfg, P, theta=None):
     return reach.astype(bool), itv, state, j, e
 
 
+def symik_vs_oracle(hs, oracle, name, cfg, ocfg, P, ill=None, theta=None):
+    """hs_symik against oracle.symik_batch on the same poses: a Report with flags, states, intervals, joints and elbows
+    (the caller checks it), and the oracle's outputs."""
+    want = oracle.symik_batch(ocfg, P, theta)
+    reach, itv, state, joints, elbow = hs_symik(hs, cfg, P, theta)
+    rep = Report(name, len(P), ill)
+    rep.exact("reachable", reach, want[0])
+    rep.exact("state", state, want[2])
+    rep.close("interval", itv, want[1])
+    rep.close("joints", joints, want[3])
+    rep.close("elbow", elbow, want[4])
+    return rep, state, want
+
+
+def hs_no_limits(hs, cfg, P, theta):
+    P = np.ascontiguousarray(P, dtype=np.float64)
+    n = len(P)
+    kind = _abi.POSE_MAT4 if P.shape[1:] == (4, 4) else _abi.POSE_EULER6
+    nj = np.empty((n, 7)); ne = np.empty((n, 3))
+    hs.hs_no_limits_batch(C.byref(cfg), kind, dp(P), dp(np.ascontiguousarray(theta, dtype=np.float64)), C.c_int64(n), dp(nj), dp(ne))
+    return nj, ne
+
+
+def hs_ctl_discrete(hs, cfg, par, M, prev, cur=None, compact=False):
+    """The discrete controller on (n,4,4) goals: one pass per pose (r2ik_ctl_discrete_f64) or the classify / search /
+    finish passes over compacted lists (r2ik_ctl_discrete_compact_f64).  Returns joints, reachable, state, emergency."""
+    M = np.ascontiguousarray(M, dtype=np.float64)
+    n = len(M)
+    cur = prev if cur is None else cur
+    joints = np.empty((n, 7)); reach = np.zeros(n, np.uint8); state = np.zeros(n, np.uint8); emg = np.zeros(n, np.uint8)
+    if compact:
+        lists = np.zeros(3, np.int64)
+        hs.hs_ctl_discrete_compact_batch(C.byref(cfg), C.byref(par), dp(M), C.c_int64(n), dp(prev), dp(cur), C.c_int(0), dp(joints),
+                                         u8(reach), u8(state), u8(emg), lists.ctypes.data_as(C.POINTER(C.c_int64)))
+    else:
+        hs.hs_ctl_discrete_batch(C.byref(cfg), C.byref(par), dp(M), C.c_int64(n), dp(prev), dp(cur), dp(joints), u8(reach),
+                                 u8(state), u8(emg))
+    return joints, reach.astype(bool), state, emg
+
+
 def urdf_params():
     u = load("symik_urdf.npz")
     return {k[len("param_"):]: u[k] for k in u.files if k.startswith("param_")}
@@ -197,10 +237,7 @@ def test_urdf_and_no_limits(hs, oracle, arm):
     rep.exact("state", state, g[f"{arm}_state"])
     rep.close("interval", itv, g[f"{arm}_interval"])
     rep.close("joints", joints, g[f"{arm}_joints"])
-    n = len(M)
-    nj = np.empty((n, 7)); ne = np.empty((n, 3))
-    Mc = np.ascontiguousarray(M)
-    hs.hs_no_limits_batch(C.byref(cfg), _abi.POSE_MAT4, dp(Mc), dp(np.ascontiguousarray(th)), C.c_int64(n), dp(nj), dp(ne))
+    nj, ne = hs_no_limits(hs, cfg, M, th)
     rep.close("no_limits joints", nj, g[f"{arm}_nl_joints"])
     rep.close("no_limits elbow", ne, g[f"{arm}_nl_elbow"])
     rep.check()
@@ -231,11 +268,9 @@ def test_ctl_discrete(hs, oracle, arm, variant):
     par = ctl_params(oracle, arm, **kw)
     n = len(M)
     prev = np.array(oracle.DEFAULT_PREV_JOINTS[arm])
-    joints = np.empty((n, 7)); reach = np.zeros(n, np.uint8); state = np.zeros(n, np.uint8); emg = np.zeros(n, np.uint8)
-    hs.hs_ctl_discrete_batch(C.byref(cfg), C.byref(par), dp(M), C.c_int64(n), dp(prev), dp(prev), dp(joints), u8(reach),
-                             u8(state), u8(emg))
+    joints, reach, state, emg = hs_ctl_discrete(hs, cfg, par, M, prev)
     rep = Report(f"hostsim ctl discrete {arm} {variant}", n, ill)
-    rep.exact("reachable", reach.astype(bool), want_f)
+    rep.exact("reachable", reach, want_f)
     rep.exact("state", state, want_s)
     rep.close("joints", joints, want_j)
     rep.check(max_ill_fraction=0.02)
@@ -773,12 +808,7 @@ def test_non_orthonormal_rotation_blocks(hs, oracle, kind):
     X = M.astype(np.float32).astype(np.float64) if kind == "float32_rounded" else np.round(M, 5)
     ocfg = oracle.arm_config("r_arm")
     ill = ill_conditioned_mask(lambda p: oracle.symik_batch(ocfg, p.reshape(X.shape))[:4], X.reshape(len(X), -1), n_trials=2)
-    want = oracle.symik_batch(ocfg, X)
-    reach, itv, state, joints, elbow = hs_symik(hs, cfg_for("r_arm"), X)
-    rep = Report(f"hostsim non-orthonormal {kind}", len(X), ill)
-    rep.exact("state", state, want[2])
-    rep.close("interval", itv, want[1])
-    rep.close("joints", joints, want[3])
+    rep = symik_vs_oracle(hs, oracle, f"hostsim non-orthonormal {kind}", cfg_for("r_arm"), ocfg, X, ill)[0]
     rep.check(max_ill_fraction=0.03)   # FK-sampled poses reach down to a straight arm: ~1.7 % move by > 1e-10 under 3e-13
 
 
@@ -876,3 +906,43 @@ def test_ctl_discrete_three_passes_equal_one_pass(hs, oracle, arm, variant):
             assert int(three[1].sum()) == lists[1] and int((three[2] == 9).sum()) == len(M[::97])
             n_literal += int(lists[2])
     assert n_literal > 0, "no pose of the sample took the literal solve: the flag path of the finish pass was not exercised"
+
+
+@pytest.mark.parametrize("arm", ARMS)
+def test_edge_inputs(hs, oracle, arm):
+    """The extreme families of tests/edge_inputs.py (goals at 10^-300 .. 10^200 m, wrists within 10^-300 m of the
+    shoulder, rotation blocks scaled by 10^-100 .. 10^100, signed zeros, subnormal entries, rotation_matrix_from_vector
+    edges, non-orthonormal blocks, euler angles up to 1e15 rad) through the kernel source on the host, with the helpers
+    the golden tests above use: FP64 solve, no-limits solve, and the discrete controller (one pass and compacted
+    passes, matrix families only), against the oracle.  test_gpu_edges.py runs the same families on the device.
+    (The scalar entry's per-call body lives in the kernel file, not in a shared header: it is run on the device only.)"""
+    import edge_inputs as E
+
+    cfg, ocfg = cfg_for(arm), oracle.arm_config(arm)
+    params = urdf_params()
+    ccfg, cocfg = cfg_for(arm, params, -1.01), oracle.arm_config(arm, ik_parameters=params, singularity_offset=-1.01)
+    par, opar = ctl_params(oracle, arm), oracle.ControlParams(arm=arm)
+    prev = np.array(oracle.DEFAULT_PREV_JOINTS[arm])
+    rng = np.random.default_rng(3)
+    for name, P in {**E.mat4_families(arm), **E.euler_families(arm)}.items():
+        ill = E.undetermined_wrist_direction(arm, P) if name == "near_shoulder" else None
+        rep, state, want = symik_vs_oracle(hs, oracle, f"hostsim edges {name} {arm}", cfg, ocfg, P, ill)
+        th = E.big_thetas(len(P))
+        rep.close("joints@big theta", hs_symik(hs, cfg, P, th)[3], oracle.symik_batch(ocfg, P, th)[3])
+        th = np.where(rng.random(len(P)) < 0.5, rng.uniform(-np.pi, np.pi, len(P)), E.big_thetas(len(P)))
+        nj, ne = hs_no_limits(hs, cfg, P, th)
+        wj, we = oracle.symik_no_limits_batch(ocfg, P, th)
+        rep.close("no_limits joints", nj, wj)
+        rep.close("no_limits elbow", ne, we)
+        dstates = []
+        if P.shape[1:] == (4, 4):
+            wj, wr, ws, we = oracle.ctl_discrete_batch(cocfg, opar, P)
+            for compact in (False, True):
+                j, r, st, emg = hs_ctl_discrete(hs, ccfg, par, P, prev, compact=compact)
+                rep.exact(f"discrete{' compact' if compact else ''} emergency", emg, we)
+                rep.exact(f"discrete{' compact' if compact else ''} reachable", r, wr)
+                rep.exact(f"discrete{' compact' if compact else ''} state", st, ws)
+                rep.close(f"discrete{' compact' if compact else ''} joints", j, wj)
+                dstates.append((st, ws))
+        rep.check(max_ill_fraction=1.0 if ill is not None else 0.0)
+        assert np.array_equal(state, want[2]) and all(np.array_equal(a, b) for a, b in dstates), rep.summary()

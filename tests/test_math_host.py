@@ -1,9 +1,12 @@
 """r2ik_math.cuh on the host: accuracy and IEEE special cases of the straight-line atan2 that the
-kernels use instead of the CUDA library routine (same source; the host build divides with '/'
-where the device uses the MUFU seed + Newton steps, which the GPU parity tests cover)."""
+kernels use instead of the CUDA library routine.  The host build takes the exact library operation
+wherever the source branches on __CUDA_ARCH__ ('/' and sqrt where the device uses a MUFU seed + Newton
+steps), so these tests check the polynomials and the octant logic only; the device arithmetic itself
+is compared with references in tests/test_gpu_math.py."""
 import ctypes as C
 import math
 import os
+import re
 import subprocess
 
 import numpy as np
@@ -127,3 +130,55 @@ def test_sincos_small_vs_mpmath(hs):
             worst = max(worst, float(abs(mp.mpf(float(got)) - want)) / (scale * 2.0 ** -52))
     assert worst < 2.0, worst
     assert np.max(np.abs(sn - np.sin(x))) < 3e-16 and np.max(np.abs(cs - np.cos(x))) < 3e-16
+
+
+# Every call of the math routines whose domain has no validity predicate, with the reason its argument is inside the
+# domain.  div_fast / rcp_fast: 2^-1022 <= |divisor| < 2^1022 (rcp.approx.ftz flushes a smaller reciprocal to zero);
+# sqrt_nonneg / sqrt_rsqrt_nonneg: +-0 or a finite normal number (the root of +inf is NaN on the device).  A new call
+# site fails this test until its argument has been argued into the domain here.
+GUARDED_CALLS = {
+    ("r2ik_math.cuh", "div_fast(num, den)"): "atan2_core: atan2_core_ok keeps den = mx or mn + mx below 2^1022",
+    ("r2ik_device.cuh", "div_fast(1.0 - ux, uy * uy + uz * uz)"): "rmfv_columns: unit vector, not within isclose of +-e_x",
+    ("r2ik_device.cuh", "div_fast(d_target, fabs(d) + A.proj_margin)"): "reduce_goal: d = |w - s| of a projected goal, >= margin",
+    ("r2ik_device.cuh", "div_fast(A.max_arm_length, sqrt_nonneg(dg2) + A.proj_margin)"): "reach_prechecks: dg2 < inf tested",
+    ("r2ik_device.cuh", "rcp_fast(2.0 * qa)"): "literal circle intersection: qa = |v|^2 of a unit direction",
+    ("r2ik_device_f32.cuh", "div_fast(A64.d_min, d + A64.proj_margin)"): "FP32 front end: d < d_min, >= margin",
+    ("r2ik_control.cuh", "sqrt_nonneg(cross ? s2 : 0.0)"): "interval plan: s2 = R^2 - C^2 of unit-scale coefficients",
+    ("r2ik_device.cuh", "sqrt_nonneg(q12 * q12 + q22 * q22)"): "orbita3d clamp: entries of a rotation, <= 1",
+    ("r2ik_device.cuh", "sqrt_nonneg(rad)"): "elbow_circle: negative rad is NaN by the select; |rad| <= 4 d^2 L1^2",
+    ("r2ik_device.cuh", "sqrt_nonneg(dg2)"): "reach_prechecks: under the dg2 < inf test",
+    ("r2ik_device.cuh", "sqrt_rsqrt_nonneg(dx * dx + dy * dy + dz * dz, invd)"):
+        "solve_core: |w - s|^2 is finite (goal inside the reach sphere, orthonormal rotation); a wrist within ~1.5e-154 m "
+        "of the shoulder gives a subnormal square and an inexact d, but then d < d_min: reduce_goal divides by "
+        "|d| + proj_margin and d is recomputed from the pushed-out wrist",
+    ("r2ik_device.cuh", "sqrt_nonneg(dl)"): "fast circle linking: dl >= 0 in that branch, O(1)",
+    ("r2ik_device.cuh", "sqrt_nonneg(disc)"): "literal circle intersection: disc >= 0 in that branch, O(1)",
+    ("r2ik_device_f32.cuh", "sqrt_rsqrt_nonneg(d2, invd64)"):
+        "FP32 front end / reach map: 0 <= d2 < d_min^2; a subnormal d2 (wrist within ~1.5e-154 m of the shoulder) "
+        "gives an inexact d, but such a pose is escalated (d2 <= 1e-12) and only |d| + proj_margin divides",
+}
+
+
+def test_call_sites_of_unguarded_routines():
+    """The device calls of div_fast, rcp_fast, sqrt_nonneg and sqrt_rsqrt_nonneg are exactly the ones listed in
+    GUARDED_CALLS (test_gpu_math.py measures the routines inside their domains)."""
+    csrc = os.path.join(REPO, "reachy2_symbolic_ik_b200", "csrc")
+    call = re.compile(r"\b(div_fast|rcp_fast|sqrt_nonneg|sqrt_rsqrt_nonneg)\(")
+    found = set()
+    for f in sorted(os.listdir(csrc)):
+        if not f.endswith((".cuh", ".cu")):
+            continue
+        for line in open(os.path.join(csrc, f)):
+            code = line.split("//")[0]
+            if "R2IK_HD" in code:
+                continue                                   # the definitions
+            for m in call.finditer(code):
+                depth, k = 0, m.end() - 1
+                while True:                                # the call up to its closing parenthesis
+                    depth += {"(": 1, ")": -1}.get(code[k], 0)
+                    if depth == 0:
+                        break
+                    k += 1
+                found.add((f, code[m.start():k + 1]))
+    assert found == set(GUARDED_CALLS), (f"unlisted: {sorted(found - set(GUARDED_CALLS))}\n"
+                                         f"gone: {sorted(set(GUARDED_CALLS) - found)}")
