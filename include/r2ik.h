@@ -19,6 +19,10 @@
  *   r2ik_elbow_positions_f64
  *        SymbolicIK.get_elbow_position             symbolic_ik.py:684-695
  *        (on the circle stored by is_reachable :197 or by is_reachable_no_limits :114-116)
+ *   r2ik_symik_sweep_f64
+ *        theta_to_joints_func called at K elbow angles per pose
+ *                                                  symbolic_ik.py:121-282, 85-119, 697-863
+ *        (angles placed like get_best_discrete_theta utils.py:366-375)
  *   r2ik_symik_scalar_f64
  *        the scalar call sequence is_reachable / is_reachable_no_limits -> get_elbow_position
  *        -> get_joints of ONE pose in one launch   symbolic_ik.py:121-282, 85-119, 684-695, 697-863
@@ -69,7 +73,7 @@
 extern "C" {
 #endif
 
-#define R2IK_ABI_VERSION 4 /* 4: + ctl_discrete_compact; 3: + symik_scalar, stream_synchronize, host pipelines, ctl_ctor_theta, reach_map_range_u16; no_limits / projected in elbow_positions, prev_joints in
+#define R2IK_ABI_VERSION 5 /* 5: + symik_sweep; 4: + ctl_discrete_compact; 3: + symik_scalar, stream_synchronize, host pipelines, ctl_ctor_theta, reach_map_range_u16; no_limits / projected in elbow_positions, prev_joints in
                               no_limits, nullable `reachable`, test hook of the phased continuous entry as a parameter */
 
 /* argument errors */
@@ -94,7 +98,7 @@ extern "C" {
 #define R2IK_POSE_EULER6 0 /* n x 6 : x y z roll pitch yaw  (the reference's goal_pose, 2x3)     */
 #define R2IK_POSE_MAT4 1   /* n x 16: row-major 4x4; converted like control_ik.py:216 (no snap) */
 #define R2IK_POSE_MAT34 2  /* n x 12: the 3x4 top of that matrix (the last row is never read);    */
-                           /*   r2ik_symik_solve_f64 only                                          */
+                           /*   r2ik_symik_solve_f64 and r2ik_symik_sweep_f64 only                 */
 
 /* emergency reason bits (utils.py:544-566, 584-586) */
 #define R2IK_EMG_SHOULDER_PITCH 1
@@ -237,6 +241,24 @@ int r2ik_symik_no_limits_f64(r2ik_handle h, int pose_kind, const double *poses, 
 int r2ik_elbow_positions_f64(r2ik_handle h, int pose_kind, const double *poses, const double *thetas,
                              int32_t K, int64_t n, int32_t no_limits, double *elbows /* n*K*3 */,
                              uint8_t *projected, void *stream);
+
+/* Elbow-angle sweep: for every pose i and sample k < K, is_reachable(poses[i]) (no_limits = 1: is_reachable_no_limits)
+ * followed by get_joints(theta_ik, previous_joints) as the FIRST call on that solve (symbolic_ik.py:121-282, 85-119,
+ * 697-863) -- bit-identical to r2ik_symik_solve_f64 (r2ik_symik_no_limits_f64) on the pose repeated K times with the
+ * flattened angles.  The pose is solved once per tile of up to 1 024 of its samples.  The reference's closure, called
+ * repeatedly on one solver, leaks state from one call to the next (once the elbow projection fires, later calls see a
+ * shifted goal); like r2ik_symik_solve_f64 this entry does not reproduce that leak.
+ * Angles: thetas non-NULL: row i at thetas + i * theta_stride, theta_stride = K (one row per pose) or 0 (one row of K
+ * shared by all poses).  thetas NULL: K samples on each pose's theta_interval, placed as get_best_discrete_theta places
+ * them (utils.py:366-375): linspace(pi/2, 5pi/2, K) for a full circle, a wrapped interval unrolled by +2pi.
+ * A pose that is not reachable ("limited by wrist" included) gets NaN thetas_used / joints / elbow and projected = 0 for
+ * all K samples.  state: n; interval: n x 2, nullable; thetas_used (the angles used): n x K, nullable; joints:
+ * n x K x 7; elbow: n x K x 3, nullable (get_joints' elbow); projected: n x K, nullable, 1 where make_elbow_projection
+ * fired.  prev_joints: nullable, 7 doubles broadcast (NULL = zeros).  K >= 1; n * K * 7 must fit int64. */
+int r2ik_symik_sweep_f64(r2ik_handle h, int pose_kind, const double *poses, int64_t n, const double *thetas,
+                         int32_t theta_stride, int32_t K, int32_t no_limits, const double *prev_joints, uint8_t *state,
+                         double *interval, double *thetas_used, double *joints, double *elbow, uint8_t *projected,
+                         void *stream);
 
 /* The scalar call sequence of SymbolicIK for one pose in one launch.  query: HOST pointer (passed to the kernel by
  * value).  out: any device-accessible address -- device memory, or pinned host memory (cudaHostAlloc / torch

@@ -6,7 +6,7 @@ import ctypes as C
 
 import numpy as np
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 POSE_EULER6 = 0
 POSE_MAT4 = 1

@@ -26,7 +26,7 @@ def use_library(path: str) -> None:
 EXPORTS = (
     "r2ik_abi_version", "r2ik_last_error", "r2ik_create", "r2ik_destroy", "r2ik_get_constants",
     "r2ik_interval_limit", "r2ik_symik_solve_f64", "r2ik_symik_solve_f32", "r2ik_symik_no_limits_f64", "r2ik_elbow_positions_f64",
-    "r2ik_symik_scalar_f64", "r2ik_stream_synchronize", "r2ik_ctl_ctor_theta_f64",
+    "r2ik_symik_sweep_f64", "r2ik_symik_scalar_f64", "r2ik_stream_synchronize", "r2ik_ctl_ctor_theta_f64",
     "r2ik_ctl_discrete_f64", "r2ik_ctl_discrete_scan_f64", "r2ik_ctl_discrete_compact_f64", "r2ik_ctl_discrete_workspace_bytes", "r2ik_ctl_continuous_f64", "r2ik_ctl_continuous_phased_f64", "r2ik_reach_map_u32", "r2ik_reach_map_f64_u32", "r2ik_reach_map_range_u16", "r2ik_fk_f64", "r2ik_copy2d_async",
     "r2ik_dfma_probe", "r2ik_ffma_probe",
     "r2ik_pipeline_create", "r2ik_pipeline_destroy", "r2ik_pipeline_wait", "r2ik_pipeline_last_error", "r2ik_pipeline_symik_f64",
@@ -63,6 +63,7 @@ def load() -> C.CDLL:
     L.r2ik_symik_solve_f32.argtypes = [vp, C.c_int, vp, vp, vp, i64, vp, vp, vp, vp, vp, vp, vp, vp]
     L.r2ik_symik_no_limits_f64.argtypes = [vp, C.c_int, vp, vp, vp, i32, i64, vp, vp, vp, vp]
     L.r2ik_elbow_positions_f64.argtypes = [vp, C.c_int, vp, vp, i32, i64, i32, vp, vp, vp]
+    L.r2ik_symik_sweep_f64.argtypes = [vp, C.c_int, vp, i64, vp, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp]
     L.r2ik_symik_scalar_f64.argtypes = [vp, C.POINTER(_abi.ScalarQuery), vp, vp]
     L.r2ik_stream_synchronize.argtypes = [vp]
     L.r2ik_ctl_ctor_theta_f64.argtypes = [vp, C.c_double, C.POINTER(C.c_double), i32, C.POINTER(C.c_double), vp, vp]

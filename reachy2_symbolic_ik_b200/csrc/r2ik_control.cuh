@@ -8,14 +8,6 @@
 
 namespace r2ik {
 
-// Sampling range of get_best_discrete_theta (utl:366-375): full circle uses a vertical
-// symmetry [pi/2, 5pi/2]; a wrapped interval is unrolled past pi.
-R2IK_HD void search_range(double i0, double i1, double &start, double &stop) {
-  if (fabs(fabs(i0) + fabs(i1) - kTwoPi) < 0.00001) { start = kHalfPi; stop = kHalfPi + kTwoPi; }
-  else if (i0 < i1) { start = i0; stop = i1; }
-  else { start = i0; stop = i1 + kTwoPi; }
-}
-
 // is_elbow_ok(get_elbow_position(theta)) (utl:443-465 on sik:684-695) as two half-plane tests in
 // (cos theta, sin theta): the elbow point is c + a1 r cos + a2 r sin, and both conditions of the
 // predicate are linear in it:

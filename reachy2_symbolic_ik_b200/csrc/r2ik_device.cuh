@@ -195,6 +195,14 @@ R2IK_HD double linspace_value(const Linspace &L, int i) {
   return mul_add_unfused((double)i, L.step, L.start);
 }
 
+// Sampling range of get_best_discrete_theta (utl:366-375): full circle uses a vertical
+// symmetry [pi/2, 5pi/2]; a wrapped interval is unrolled past pi.
+R2IK_HD void search_range(double i0, double i1, double &start, double &stop) {
+  if (fabs(fabs(i0) + fabs(i1) - kTwoPi) < 0.00001) { start = kHalfPi; stop = kHalfPi + kTwoPi; }
+  else if (i0 < i1) { start = i0; stop = i1; }
+  else { start = i0; stop = i1 + kTwoPi; }
+}
+
 // ---------------------------------------------------------------------------------------
 // scipy Rotation, quaternion (x, y, z, w)
 // ---------------------------------------------------------------------------------------
@@ -1121,13 +1129,14 @@ R2IK_HD bool load_pose(const double *row, bool snap, double pos[3], double R[9])
 // ---------------------------------------------------------------------------------------
 // Per-pose bodies of the SymbolicIK kernels (r2ik_kernels.cu; tests/hostsim loops over the same functions)
 // ---------------------------------------------------------------------------------------
-// K1, solve: is_reachable on a pose row (INVALID_ROTATION with a NaN interval for det <= 0).
-template <int KIND>
+// K1, solve: is_reachable (NO_LIMITS: is_reachable_no_limits) on a pose row (INVALID_ROTATION with a NaN interval for
+// det <= 0).
+template <int KIND, bool NO_LIMITS = false>
 R2IK_HD Reach symik_reach(const ArmConst &A, const double *row, Solve &S) {
   double pos[3];
   Reach rc;
   rc.state = R2IK_STATE_INVALID_ROTATION; rc.i0 = NAN; rc.i1 = NAN;
-  if (load_pose<KIND>(row, false, pos, S.R)) rc = is_reachable_R<false>(A, pos, S);
+  if (load_pose<KIND>(row, false, pos, S.R)) rc = is_reachable_R<NO_LIMITS>(A, pos, S);
   return rc;
 }
 
@@ -1184,6 +1193,36 @@ R2IK_HD bool pose_elbow_circle(const ArmConst &A, const double *row, Solve &S) {
     ok = st == R2IK_STATE_REACHABLE || (!NO_LIMITS && st == R2IK_STATE_LIMITED_BY_WRIST);
   }
   return ok;
+}
+
+// Elbow-angle sweep (k_symik_sweep): angle k of K for a pose solved by symik_reach.  row: the pose's K given angles, or
+// null for K samples placed on theta_interval as get_best_discrete_theta places them (utl:366-375).  NaN for a pose
+// that is not reachable.
+R2IK_HD double sweep_theta(const Reach &rc, const double *row, int K, int k) {
+  if (rc.state != R2IK_STATE_REACHABLE) return NAN;
+  if (row) return row[k];
+  double start, stop;
+  search_range(rc.i0, rc.i1, start, stop);
+  return linspace_value(make_linspace(start, stop, K), k);
+}
+
+// One sample of the sweep: get_joints(theta) as the first call on the pose's solve S0 -- the value K1 (K1b) returns for
+// the same pose and theta.  get_joints moves S.p / S.w when the elbow projection fires, so every sample starts from its
+// own copy of S0.  NaN for a pose that is not reachable.  Returns whether the elbow projection fires at theta.
+R2IK_HD bool sweep_sample(const ArmConst &A, const Solve &S0, const Reach &rc, double theta, double prev0, double prev2,
+                          double j[7], double E[3]) {
+  if (rc.state != R2IK_STATE_REACHABLE) {
+    for (int k = 0; k < 7; ++k) j[k] = NAN;
+    E[0] = NAN; E[1] = NAN; E[2] = NAN;
+    return false;
+  }
+  Solve S = S0;
+  double st, ct, Ep[3];
+  sincos_any(theta, st, ct);
+  elbow_position_cs(S, ct, st, Ep);
+  const bool proj = elbow_projection_fires(A, Ep);
+  get_joints_cs(A, S, ct, st, prev0, prev2, j, E);
+  return proj;
 }
 
 // get_elbow_position(*theta) on that circle (NaN without one).  Returns whether the elbow projection fires there.

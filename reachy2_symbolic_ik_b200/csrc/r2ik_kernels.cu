@@ -3,6 +3,7 @@
 //   K1     k_symik_solve                        one thread / pose: is_reachable + get_joints (FP64)
 //   K1-f32 k_symik_solve_f32 + k_symik_escalated_f32   the FP32 fast path; undecidable poses re-solved in FP64
 //   K1b    k_symik_no_limits, k_elbow_positions    is_reachable_no_limits, get_elbow_position
+//   K1s    k_symik_sweep                        one solve per pose, get_joints at K elbow angles spread over the block
 //   K2     k_ctl_discrete                       one lane / pose, analytic arg-min over the K elbow samples
 //          k_ctl_discrete_scan                  the exhaustive warp-cooperative scan of the K samples (cross-check)
 //   K3     k_cont_targets / k_cont_thetas / k_cont_raw_joints_codes / k_cont_finish_codes / k_cont_apply_windings
@@ -203,6 +204,60 @@ k_elbow_positions(const __grid_constant__ ArmConst A, const double *__restrict__
     double *o = elbows + ((size_t)i * K + k) * 3;
     o[0] = E[0]; o[1] = E[1]; o[2] = E[2];
     if (projected) projected[(size_t)i * K + k] = proj ? 1 : 0;
+  }
+}
+
+// ---------------------------------------------------------------------------------------
+// K1s: elbow-angle sweep, get_joints at K angles per pose from one solve of the pose.
+// A block owns a tile of P poses x Kt samples (sweep_tile): threads < P solve one pose each and leave its Solve and
+// Reach in shared memory, then the block walks the P * Kt items pose-major, sample-minor, so consecutive threads store
+// consecutive 56-byte joint rows.  A pose whose K samples span several tiles is solved once per tile.
+// ---------------------------------------------------------------------------------------
+// 4 blocks / SM (128 registers, ~145 B of spills): 10-28 % faster than 2 blocks at 255 registers without spills on every
+// shape of scripts/experiments/exp_sweep.py (profiles/r3_exp_sweep*.txt)
+#ifndef R2IK_K1S_MINBLOCKS
+#define R2IK_K1S_MINBLOCKS 4
+#endif
+template <int KIND, bool NO_LIMITS>
+__global__ void __launch_bounds__(R2IK_BLOCK, R2IK_K1S_MINBLOCKS)
+k_symik_sweep(const __grid_constant__ ArmConst A, const double *__restrict__ poses, int64_t n, const double *__restrict__ thetas,
+              int theta_stride, int K, int P, int Kt, int n_ktiles, const double *__restrict__ prev_joints,
+              uint8_t *__restrict__ state, double *__restrict__ interval, double *__restrict__ thetas_used,
+              double *__restrict__ joints, double *__restrict__ elbow, uint8_t *__restrict__ projected) {
+  __shared__ Solve sS[R2IK_BLOCK];
+  __shared__ Reach sR[R2IK_BLOCK];
+  asm volatile("griddepcontrol.launch_dependents;");
+  asm volatile("griddepcontrol.wait;" ::: "memory");
+  double prev0 = 0.0, prev2 = 0.0;
+  if (prev_joints) { prev0 = prev_joints[0]; prev2 = prev_joints[2]; }
+  const int64_t p0 = (int64_t)(blockIdx.x / n_ktiles) * P;
+  const int kt = (int)(blockIdx.x % n_ktiles), k0 = kt * Kt;
+  const int np = (int)min((int64_t)P, n - p0), nk = min(Kt, K - k0);
+  if (threadIdx.x < np) {
+    const int64_t i = p0 + threadIdx.x;
+    Solve S;
+    const Reach rc = symik_reach<KIND, NO_LIMITS>(A, poses + pose_stride(KIND) * i, S);
+    sS[threadIdx.x] = S;
+    sR[threadIdx.x] = rc;
+    if (kt == 0) {
+      state[i] = (uint8_t)rc.state;
+      if (interval) { interval[2 * i] = rc.i0; interval[2 * i + 1] = rc.i1; }
+    }
+  }
+  __syncthreads();
+  for (int f = threadIdx.x; f < np * nk; f += blockDim.x) {
+    const int p = f / nk, k = k0 + (f - p * nk);
+    const int64_t i = p0 + p;
+    const Reach rc = sR[p];
+    const double th = sweep_theta(rc, thetas ? thetas + (size_t)theta_stride * i : nullptr, K, k);
+    double j[7], E[3];
+    const bool proj = sweep_sample(A, sS[p], rc, th, prev0, prev2, j, E);
+    const size_t o = (size_t)i * K + k;
+#pragma unroll
+    for (int q = 0; q < 7; ++q) joints[7 * o + q] = j[q];
+    if (elbow) { elbow[3 * o] = E[0]; elbow[3 * o + 1] = E[1]; elbow[3 * o + 2] = E[2]; }
+    if (thetas_used) thetas_used[o] = th;
+    if (projected) projected[o] = proj ? 1 : 0;
   }
 }
 
@@ -771,6 +826,18 @@ struct DeviceGuard {
 static inline bool misaligned16(const void *p) { return ((uintptr_t)p & 15) != 0; }
 static inline unsigned blocks_for(int64_t n) { return (unsigned)((n + R2IK_BLOCK - 1) / R2IK_BLOCK); }
 
+// Tile of k_symik_sweep: Kt samples of each of P poses, about 1024 items (8 per thread).  Few angles per pose: P = 128,
+// every thread solves a pose.  Many angles: fewer poses per tile, and while the grid would leave the 148 SMs short of
+// 8 tiles each the samples of a pose are split over more tiles (down to 128 samples a tile), each of which solves the
+// pose again.
+static void sweep_tile(int64_t n, int K, int &P, int &Kt) {
+  constexpr int kItems = 1024, kMinKt = 128;
+  constexpr int64_t kFullGrid = 148 * 8;
+  Kt = K < kItems ? K : kItems;
+  P = kItems / Kt < R2IK_BLOCK ? kItems / Kt : R2IK_BLOCK;
+  while (Kt > kMinKt && (n + P - 1) / P * ((K + Kt - 1) / Kt) < kFullGrid) Kt = (Kt + 1) / 2;
+}
+
 // Launch as a programmatic dependent of the preceding work on the stream: the kernel's blocks may be scheduled under its
 // predecessor's tail, and the kernel waits (griddepcontrol.wait) before it touches memory.
 template <typename... KArgs, typename... Args>
@@ -943,6 +1010,41 @@ int r2ik_elbow_positions_f64(r2ik_handle h, int pose_kind, const double *poses, 
     else k_elbow_positions<R2IK_POSE_EULER6, false><<<g, R2IK_BLOCK, 0, s>>>(h->A, poses, thetas, K, n, elbows, projected);
   }
   R2IK_CUDA(cudaGetLastError(), "k_elbow_positions launch");
+  return 0;
+}
+
+int r2ik_symik_sweep_f64(r2ik_handle h, int pose_kind, const double *poses, int64_t n, const double *thetas,
+                         int32_t theta_stride, int32_t K, int32_t no_limits, const double *prev_joints, uint8_t *state,
+                         double *interval, double *thetas_used, double *joints, double *elbow, uint8_t *projected,
+                         void *stream) {
+  if (n < 0 || K < 1 || (pose_kind != R2IK_POSE_EULER6 && pose_kind != R2IK_POSE_MAT4 && pose_kind != R2IK_POSE_MAT34))
+    return fail_arg(R2IK_ERR_ARG, "r2ik_symik_sweep_f64: bad n, K (>= 1) or pose_kind");
+  if (theta_stride != 0 && theta_stride != K)
+    return fail_arg(R2IK_ERR_ARG, "r2ik_symik_sweep_f64: theta_stride must be 0 (one shared row) or K (one row per pose)");
+  if (n > INT64_MAX / K / 7) return fail_arg(R2IK_ERR_ARG, "r2ik_symik_sweep_f64: n * K * 7 overflows");
+  if (!h) return fail_arg(R2IK_ERR_NULL, "r2ik_symik_sweep_f64: null handle");
+  if (n == 0) return 0;
+  if (!poses || !state || !joints) return fail_arg(R2IK_ERR_NULL, "r2ik_symik_sweep_f64: null argument");
+  if (misaligned16(poses)) return fail_arg(R2IK_ERR_ARG, "r2ik_symik_sweep_f64: poses must be 16-byte aligned");
+  DeviceGuard guard_(h->device);
+  R2IK_CUDA(guard_.err, "cudaSetDevice");
+  cudaStream_t s = (cudaStream_t)stream;
+  int P, Kt;
+  sweep_tile(n, K, P, Kt);
+  const int n_ktiles = (K + Kt - 1) / Kt;
+  const int64_t n_tiles = (n + P - 1) / P * n_ktiles;
+  if (n_tiles > 0x7fffffffLL) return fail_arg(R2IK_ERR_ARG, "r2ik_symik_sweep_f64: more than 2^31 - 1 tiles");
+  const unsigned g = (unsigned)n_tiles;
+#define R2IK_SWEEP(KIND, NL) \
+  launch_pdl(k_symik_sweep<KIND, NL>, g, R2IK_BLOCK, s, h->A, poses, n, thetas, (int)theta_stride, (int)K, P, Kt, n_ktiles, \
+             prev_joints, state, interval, thetas_used, joints, elbow, projected)
+  cudaError_t e;
+  if (pose_kind == R2IK_POSE_MAT4) e = no_limits ? R2IK_SWEEP(R2IK_POSE_MAT4, true) : R2IK_SWEEP(R2IK_POSE_MAT4, false);
+  else if (pose_kind == R2IK_POSE_MAT34) e = no_limits ? R2IK_SWEEP(R2IK_POSE_MAT34, true) : R2IK_SWEEP(R2IK_POSE_MAT34, false);
+  else e = no_limits ? R2IK_SWEEP(R2IK_POSE_EULER6, true) : R2IK_SWEEP(R2IK_POSE_EULER6, false);
+#undef R2IK_SWEEP
+  R2IK_CUDA(e, "k_symik_sweep launch");
+  R2IK_CUDA(cudaGetLastError(), "k_symik_sweep launch");
   return 0;
 }
 

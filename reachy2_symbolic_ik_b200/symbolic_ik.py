@@ -21,7 +21,7 @@ from typing import Any, Optional, Tuple
 import numpy as np
 
 from . import _abi, _native
-from .states import STATE_STRINGS
+from .states import STATE_REACHABLE, STATE_STRINGS
 
 _ZERO7 = [0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0]
 
@@ -43,6 +43,20 @@ class BatchResult:
         if hasattr(s, "cpu"):
             s = s.cpu().numpy()
         return [STATE_STRINGS[int(c)] for c in s]
+
+
+@dataclass
+class SweepResult:
+    """Outputs of ``SymbolicIK.get_joints_sweep_batch``: K elbow angles per pose.  torch CUDA tensors when the poses
+    were a CUDA tensor, NumPy arrays otherwise."""
+
+    reachable: Any        # (N,) bool
+    state: Any            # (N,) uint8, see states.STATE_STRINGS
+    theta_interval: Any   # (N, 2) float64, NaN when unreachable; [0] > [1] means wrapped
+    thetas: Any           # (N, K) float64, the angles used; NaN when unreachable
+    joints: Any           # (N, K, 7) float64, NaN when unreachable
+    elbow: Any            # (N, K, 3) float64
+    projected: Any        # (N, K) bool: make_elbow_projection fired at that angle
 
 
 def _ptr(t) -> C.c_void_p:
@@ -408,6 +422,54 @@ class SymbolicIK:
             _native.check(rc, "r2ik_symik_no_limits_f64")
             res = (joints, elbow) + ((proj.bool(),) if with_projected else ())
             return res if was_cuda else tuple(x.cpu().numpy() for x in res)
+
+    def get_joints_sweep_batch(self, poses, thetas=None, n_samples: Optional[int] = None, previous_joints=None,
+                               no_limits: bool = False) -> SweepResult:
+        """``is_reachable`` (``is_reachable_no_limits`` with ``no_limits``) of each pose, then ``theta_to_joints_func`` at K
+        elbow angles per pose, each as the first call on that solve -- the pose is solved once for its K angles.
+
+        thetas: (N,K) angles per pose, or (1,K) one row shared by all poses.  n_samples: K angles per pose placed on its
+        own theta_interval as ``get_best_discrete_theta`` places them (utils.py:366-375).  Give exactly one of the two.
+        previous_joints: None (zeros) or (7,) broadcast.  A pose that is not reachable gets NaN angles, joints and
+        elbows."""
+        if (thetas is None) == (n_samples is None):
+            raise ValueError("give either thetas (N,K) / (1,K) or n_samples, not both")
+        torch = self._torch
+        with torch.cuda.device(self._device):
+            P, kind, was_cuda = normalise_poses(torch, poses, self._device)
+            n = P.shape[0]
+            th, stride = None, 0
+            if thetas is not None:
+                th = torch.as_tensor(thetas).to(self._device, torch.float64)
+                if th.dim() != 2 or th.shape[0] not in (1, n) or th.shape[1] < 1:
+                    raise ValueError(f"thetas must be (N,K) or (1,K) with N = {n}; got {tuple(th.shape)}")
+                th = th.contiguous()
+                K = th.shape[1]
+                stride = K if th.shape[0] == n and n != 1 else 0
+            else:
+                K = int(n_samples)
+                if K < 1:
+                    raise ValueError(f"n_samples must be >= 1; got {n_samples}")
+            pj = None
+            if previous_joints is not None:
+                pj = torch.as_tensor(previous_joints).to(self._device, torch.float64).reshape(7).contiguous()
+            state = torch.empty(n, dtype=torch.uint8, device=self._device)
+            interval = torch.empty((n, 2), dtype=torch.float64, device=self._device)
+            used = torch.empty((n, K), dtype=torch.float64, device=self._device)
+            joints = torch.empty((n, K, 7), dtype=torch.float64, device=self._device)
+            elbow = torch.empty((n, K, 3), dtype=torch.float64, device=self._device)
+            proj = torch.empty((n, K), dtype=torch.uint8, device=self._device)
+            s = torch.cuda.current_stream(self._device).cuda_stream
+            rc = self._handle.lib.r2ik_symik_sweep_f64(
+                self._handle.h, kind, _ptr(P), C.c_int64(n), _ptr(th), C.c_int32(stride), C.c_int32(K),
+                C.c_int32(int(bool(no_limits))), _ptr(pj), _ptr(state), _ptr(interval), _ptr(used), _ptr(joints),
+                _ptr(elbow), _ptr(proj), C.c_void_p(s))
+            _native.check(rc, "r2ik_symik_sweep_f64")
+            res = SweepResult(state == STATE_REACHABLE, state, interval, used, joints, elbow, proj.bool())
+            if was_cuda:
+                return res
+            return SweepResult(*(x.cpu().numpy() for x in (res.reachable, res.state, res.theta_interval, res.thetas,
+                                                           res.joints, res.elbow, res.projected)))
 
     def get_elbow_position_batch(self, poses, thetas, no_limits: bool = False, with_projected: bool = False):
         """``get_elbow_position`` for K thetas per pose after ``is_reachable`` (or ``is_reachable_no_limits``): (N,K,3),
