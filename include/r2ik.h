@@ -23,6 +23,9 @@
  *        theta_to_joints_func called at K elbow angles per pose
  *                                                  symbolic_ik.py:121-282, 85-119, 697-863
  *        (angles placed like get_best_discrete_theta utils.py:366-375)
+ *   r2ik_symik_best_theta_f64
+ *        get_best_theta_to_current_joints per pose with its own current joints
+ *                                                  utils.py:267-331 on symbolic_ik.py:121-282, 85-119, 697-863
  *   r2ik_symik_scalar_f64
  *        the scalar call sequence is_reachable / is_reachable_no_limits -> get_elbow_position
  *        -> get_joints of ONE pose in one launch   symbolic_ik.py:121-282, 85-119, 684-695, 697-863
@@ -73,7 +76,7 @@
 extern "C" {
 #endif
 
-#define R2IK_ABI_VERSION 5 /* 5: + symik_sweep; 4: + ctl_discrete_compact; 3: + symik_scalar, stream_synchronize, host pipelines, ctl_ctor_theta, reach_map_range_u16; no_limits / projected in elbow_positions, prev_joints in
+#define R2IK_ABI_VERSION 6 /* 6: + symik_best_theta; 5: + symik_sweep; 4: + ctl_discrete_compact; 3: + symik_scalar, stream_synchronize, host pipelines, ctl_ctor_theta, reach_map_range_u16; no_limits / projected in elbow_positions, prev_joints in
                               no_limits, nullable `reachable`, test hook of the phased continuous entry as a parameter */
 
 /* argument errors */
@@ -98,7 +101,7 @@ extern "C" {
 #define R2IK_POSE_EULER6 0 /* n x 6 : x y z roll pitch yaw  (the reference's goal_pose, 2x3)     */
 #define R2IK_POSE_MAT4 1   /* n x 16: row-major 4x4; converted like control_ik.py:216 (no snap) */
 #define R2IK_POSE_MAT34 2  /* n x 12: the 3x4 top of that matrix (the last row is never read);    */
-                           /*   r2ik_symik_solve_f64 and r2ik_symik_sweep_f64 only                 */
+                           /*   r2ik_symik_solve_f64, _sweep_f64 and _best_theta_f64 only          */
 
 /* emergency reason bits (utils.py:544-566, 584-586) */
 #define R2IK_EMG_SHOULDER_PITCH 1
@@ -259,6 +262,20 @@ int r2ik_symik_sweep_f64(r2ik_handle h, int pose_kind, const double *poses, int6
                          int32_t theta_stride, int32_t K, int32_t no_limits, const double *prev_joints, uint8_t *state,
                          double *interval, double *thetas_used, double *joints, double *elbow, uint8_t *projected,
                          void *stream);
+
+/* The elbow angle whose joints are closest to the arm's current joints, per pose: is_reachable(poses[i]) (no_limits = 1:
+ * is_reachable_no_limits), then get_best_theta_to_current_joints(get_joints, ..., current_joints row i, arm,
+ * preferred_theta) on that solve (utils.py:267-331): the shortcut at preferred_theta (joint distance < 0.01), else a
+ * ternary search over [-pi, pi] (l_arm: [0, 2 pi]) of 16 iterations.  As in the reference, every get_joints of the search
+ * sees the goal and wrist that make_elbow_projection left behind in the previous ones (the search's order decides them).
+ * theta[i]: the reference's return value.  joints[i] (nullable, n x 7): get_joints(theta[i]) with zero previous joints as
+ * the FIRST call on a fresh solve of the pose -- bit-identical to r2ik_symik_solve_f64 (r2ik_symik_no_limits_f64) given
+ * theta[i]; the state the search leaks is not exposed.  A pose that is not reachable ("limited by wrist" included) gets
+ * NaN theta and joints.  current_joints: one row of 7 per pose (cj_stride = 7) or one row for all (cj_stride = 0).
+ * state: n. */
+int r2ik_symik_best_theta_f64(r2ik_handle h, int pose_kind, const double *poses, int64_t n, const double *current_joints,
+                              int32_t cj_stride, double preferred_theta, int32_t no_limits, uint8_t *state, double *theta,
+                              double *joints, void *stream);
 
 /* The scalar call sequence of SymbolicIK for one pose in one launch.  query: HOST pointer (passed to the kernel by
  * value).  out: any device-accessible address -- device memory, or pinned host memory (cudaHostAlloc / torch

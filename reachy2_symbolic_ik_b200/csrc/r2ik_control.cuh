@@ -224,6 +224,31 @@ R2IK_HD double best_theta_to_current_joints(const ArmConst &A, Solve &S, const d
   return best;
 }
 
+// Batched get_best_theta_to_current_joints (k_symik_best_theta): is_reachable (NO_LIMITS: is_reachable_no_limits) of a
+// pose row, then the reference's search on that solve, every get_joints seeing the goal / wrist the previous ones left
+// (best_theta_to_current_joints).  With want_joints, j = get_joints(theta) as the FIRST call on the solve -- what K1
+// (K1b) returns for that pose and theta.  get_joints moves only S.p / S.w, so those six doubles are all the fresh solve
+// needs back.  NaN theta and joints for a pose that is not reachable ("limited by wrist" included).  Returns the state.
+template <int KIND, bool NO_LIMITS>
+R2IK_HD int symik_best_theta(const ArmConst &A, const double *row, const double current_joints[7], double preferred_theta,
+                             bool want_joints, double &theta, double j[7]) {
+  Solve S;
+  const Reach rc = symik_reach<KIND, NO_LIMITS>(A, row, S);
+  if (rc.state != R2IK_STATE_REACHABLE) {
+    theta = NAN;
+    for (int k = 0; k < 7; ++k) j[k] = NAN;
+    return rc.state;
+  }
+  const double p0 = S.p[0], p1 = S.p[1], p2 = S.p[2], w0 = S.w[0], w1 = S.w[1], w2 = S.w[2];
+  theta = best_theta_to_current_joints(A, S, current_joints, preferred_theta);
+  if (want_joints) {
+    S.p[0] = p0; S.p[1] = p1; S.p[2] = p2; S.w[0] = w0; S.w[1] = w1; S.w[2] = w2;
+    double E[3];
+    get_joints(A, S, theta, 0.0, 0.0, j, E);
+  }
+  return rc.state;
+}
+
 // The same search as ControlIK's CONSTRUCTOR runs it (ctl:142-159): there `current_joints` is the list of BOTH arms' joint
 // lists, so the reference's cost loops over i < len(current_joints) = n_rows and broadcasts joints[i] against the whole
 // row i:  cost^2 = sum_{i < n_rows} sum_{k < 7} angle_diff(joints[i], rows[i][k])^2  (SURVEY.md A.6.11).  The value

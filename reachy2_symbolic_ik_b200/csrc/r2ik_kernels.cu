@@ -4,6 +4,7 @@
 //   K1-f32 k_symik_solve_f32 + k_symik_escalated_f32   the FP32 fast path; undecidable poses re-solved in FP64
 //   K1b    k_symik_no_limits, k_elbow_positions    is_reachable_no_limits, get_elbow_position
 //   K1s    k_symik_sweep                        one solve per pose, get_joints at K elbow angles spread over the block
+//   K1t    k_symik_best_theta                   one thread / pose: get_best_theta_to_current_joints (ternary search)
 //   K2     k_ctl_discrete                       one lane / pose, analytic arg-min over the K elbow samples
 //          k_ctl_discrete_scan                  the exhaustive warp-cooperative scan of the K samples (cross-check)
 //   K3     k_cont_targets / k_cont_thetas / k_cont_raw_joints_codes / k_cont_finish_codes / k_cont_apply_windings
@@ -258,6 +259,38 @@ k_symik_sweep(const __grid_constant__ ArmConst A, const double *__restrict__ pos
     if (elbow) { elbow[3 * o] = E[0]; elbow[3 * o + 1] = E[1]; elbow[3 * o + 2] = E[2]; }
     if (thetas_used) thetas_used[o] = th;
     if (projected) projected[o] = proj ? 1 : 0;
+  }
+}
+
+// ---------------------------------------------------------------------------------------
+// K1t: get_best_theta_to_current_joints, one thread / pose (symik_best_theta).  The search's range starts at 2 pi and
+// shrinks to 2/3 of itself per iteration until it is <= 0.01: 2 pi (2/3)^16 = 0.0096 < 0.01 < 2 pi (2/3)^15 = 0.0143, so
+// every lane that searches runs the same 16 iterations in lockstep, and lanes diverge only on the routes inside
+// get_joints and where a lane takes the shortcut or its pose is not reachable.
+// ---------------------------------------------------------------------------------------
+// 4 blocks / SM (128 registers, ~300 B of spills): at 1 M and 65 536 poses 13-18 % faster than 2 blocks at 198 registers
+// without spills and within 2 % of or 22 % faster than 3 blocks at 168 registers (56 B of spills)
+// (profiles/r4_exp_best_theta*.txt)
+#ifndef R2IK_K1T_MINBLOCKS
+#define R2IK_K1T_MINBLOCKS 4
+#endif
+template <int KIND, bool NO_LIMITS>
+__global__ void __launch_bounds__(R2IK_BLOCK, R2IK_K1T_MINBLOCKS)
+k_symik_best_theta(const __grid_constant__ ArmConst A, const double *__restrict__ poses, int64_t n,
+                   const double *__restrict__ current_joints, int cj_stride, double preferred_theta,
+                   uint8_t *__restrict__ state, double *__restrict__ theta, double *__restrict__ joints) {
+  asm volatile("griddepcontrol.launch_dependents;");
+  asm volatile("griddepcontrol.wait;" ::: "memory");
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  double th, j[7];
+  state[i] = (uint8_t)symik_best_theta<KIND, NO_LIMITS>(A, poses + pose_stride(KIND) * i,
+                                                        current_joints + (size_t)cj_stride * i, preferred_theta,
+                                                        joints != nullptr, th, j);
+  theta[i] = th;
+  if (joints) {
+#pragma unroll
+    for (int k = 0; k < 7; ++k) joints[7 * i + k] = j[k];
   }
 }
 
@@ -1045,6 +1078,34 @@ int r2ik_symik_sweep_f64(r2ik_handle h, int pose_kind, const double *poses, int6
 #undef R2IK_SWEEP
   R2IK_CUDA(e, "k_symik_sweep launch");
   R2IK_CUDA(cudaGetLastError(), "k_symik_sweep launch");
+  return 0;
+}
+
+int r2ik_symik_best_theta_f64(r2ik_handle h, int pose_kind, const double *poses, int64_t n, const double *current_joints,
+                              int32_t cj_stride, double preferred_theta, int32_t no_limits, uint8_t *state, double *theta,
+                              double *joints, void *stream) {
+  if (n < 0 || (pose_kind != R2IK_POSE_EULER6 && pose_kind != R2IK_POSE_MAT4 && pose_kind != R2IK_POSE_MAT34))
+    return fail_arg(R2IK_ERR_ARG, "r2ik_symik_best_theta_f64: bad n or pose_kind");
+  if (cj_stride != 0 && cj_stride != 7)
+    return fail_arg(R2IK_ERR_ARG, "r2ik_symik_best_theta_f64: cj_stride must be 0 (one shared row) or 7 (one row per pose)");
+  if (!h) return fail_arg(R2IK_ERR_NULL, "r2ik_symik_best_theta_f64: null handle");
+  if (n == 0) return 0;
+  if (!poses || !current_joints || !state || !theta) return fail_arg(R2IK_ERR_NULL, "r2ik_symik_best_theta_f64: null argument");
+  if (misaligned16(poses)) return fail_arg(R2IK_ERR_ARG, "r2ik_symik_best_theta_f64: poses must be 16-byte aligned");
+  DeviceGuard guard_(h->device);
+  R2IK_CUDA(guard_.err, "cudaSetDevice");
+  cudaStream_t s = (cudaStream_t)stream;
+  const unsigned g = blocks_for(n);
+#define R2IK_BEST_THETA(KIND, NL) \
+  launch_pdl(k_symik_best_theta<KIND, NL>, g, R2IK_BLOCK, s, h->A, poses, n, current_joints, (int)cj_stride, preferred_theta, \
+             state, theta, joints)
+  cudaError_t e;
+  if (pose_kind == R2IK_POSE_MAT4) e = no_limits ? R2IK_BEST_THETA(R2IK_POSE_MAT4, true) : R2IK_BEST_THETA(R2IK_POSE_MAT4, false);
+  else if (pose_kind == R2IK_POSE_MAT34) e = no_limits ? R2IK_BEST_THETA(R2IK_POSE_MAT34, true) : R2IK_BEST_THETA(R2IK_POSE_MAT34, false);
+  else e = no_limits ? R2IK_BEST_THETA(R2IK_POSE_EULER6, true) : R2IK_BEST_THETA(R2IK_POSE_EULER6, false);
+#undef R2IK_BEST_THETA
+  R2IK_CUDA(e, "k_symik_best_theta launch");
+  R2IK_CUDA(cudaGetLastError(), "k_symik_best_theta launch");
   return 0;
 }
 

@@ -16,7 +16,7 @@ from __future__ import annotations
 
 import ctypes as C
 from dataclasses import dataclass
-from typing import Any, Optional, Tuple
+from typing import Any, NamedTuple, Optional, Tuple
 
 import numpy as np
 
@@ -57,6 +57,16 @@ class SweepResult:
     joints: Any           # (N, K, 7) float64, NaN when unreachable
     elbow: Any            # (N, K, 3) float64
     projected: Any        # (N, K) bool: make_elbow_projection fired at that angle
+
+
+class BestThetaResult(NamedTuple):
+    """Outputs of ``SymbolicIK.get_best_theta_to_current_joints_batch``.  torch CUDA tensors when the poses were a CUDA
+    tensor, NumPy arrays otherwise."""
+
+    reachable: Any        # (N,) bool
+    state: Any            # (N,) uint8, see states.STATE_STRINGS
+    theta: Any            # (N,) float64, NaN when unreachable
+    joints: Any           # (N, 7) float64 (None without want_joints), NaN when unreachable
 
 
 def _ptr(t) -> C.c_void_p:
@@ -470,6 +480,44 @@ class SymbolicIK:
                 return res
             return SweepResult(*(x.cpu().numpy() for x in (res.reachable, res.state, res.theta_interval, res.thetas,
                                                            res.joints, res.elbow, res.projected)))
+
+    def get_best_theta_to_current_joints_batch(self, poses, current_joints, preferred_theta: Optional[float] = None,
+                                               no_limits: bool = False, want_joints: bool = True) -> BestThetaResult:
+        """``get_best_theta_to_current_joints`` (utils.py:267-331) for N poses: ``is_reachable`` (``is_reachable_no_limits``
+        with ``no_limits``) of each pose, then the reference's search for the elbow angle whose joints are closest to that
+        pose's current joints, on that solve and in the reference's order (so the state that ``get_joints`` leaks from
+        one evaluation to the next when the elbow projection fires is part of the answer, as in the reference).
+
+        current_joints: (7,) shared by all poses, or (N,7).  preferred_theta: the angle tried first; default ControlIK's
+        for this arm (-2 pi / 3 for r_arm, -pi / 3 for l_arm).  joints: get_joints(theta) as the first call on a fresh
+        solve of the pose, what ``is_reachable_batch(poses, theta)`` returns.  A pose that is not reachable gets NaN
+        theta and joints."""
+        if preferred_theta is None:
+            preferred_theta = -4 * np.pi / 6 if self.arm == "r_arm" else -np.pi - (-4 * np.pi / 6)
+        torch = self._torch
+        with torch.cuda.device(self._device):
+            P, kind, was_cuda = normalise_poses(torch, poses, self._device)
+            n = P.shape[0]
+            cj = torch.as_tensor(current_joints).to(self._device, torch.float64)
+            if cj.shape == (7,) or cj.shape == (1, 7):
+                stride = 0
+            elif cj.dim() == 2 and cj.shape == (n, 7):
+                stride = 7
+            else:
+                raise ValueError(f"current_joints must be (7,) or (N,7) with N = {n}; got {tuple(cj.shape)}")
+            cj = cj.contiguous()
+            state = torch.empty(n, dtype=torch.uint8, device=self._device)
+            theta = torch.empty(n, dtype=torch.float64, device=self._device)
+            joints = torch.empty((n, 7), dtype=torch.float64, device=self._device) if want_joints else None
+            s = torch.cuda.current_stream(self._device).cuda_stream
+            rc = self._handle.lib.r2ik_symik_best_theta_f64(
+                self._handle.h, kind, _ptr(P), C.c_int64(n), _ptr(cj), C.c_int32(stride), C.c_double(float(preferred_theta)),
+                C.c_int32(int(bool(no_limits))), _ptr(state), _ptr(theta), _ptr(joints), C.c_void_p(s))
+            _native.check(rc, "r2ik_symik_best_theta_f64")
+            res = BestThetaResult(state == STATE_REACHABLE, state, theta, joints)
+            if was_cuda:
+                return res
+            return BestThetaResult(*(None if x is None else x.cpu().numpy() for x in res))
 
     def get_elbow_position_batch(self, poses, thetas, no_limits: bool = False, with_projected: bool = False):
         """``get_elbow_position`` for K thetas per pose after ``is_reachable`` (or ``is_reachable_no_limits``): (N,K,3),
