@@ -47,6 +47,9 @@
  *        grid sweep of is_reachable (shape of src/benchmark/ik_comparison.py:137-181)
  *   r2ik_reach_map_f64_u32
  *        the same volume, every pair by the all-FP64 flag solve (cross-check)
+ *   r2ik_ctl_reach_map_u32
+ *        grid sweep of ControlIK.symbolic_inverse_kinematics(name, M, "discrete")'s `reachable`
+ *                                                  control_ik.py:162-274, 409-462 (utils.py:334-396)
  *   r2ik_interval_limit
  *        interval_limit + l_arm mirroring          control_ik.py:225-252
  *   r2ik_ctl_ctor_theta_f64
@@ -76,7 +79,7 @@
 extern "C" {
 #endif
 
-#define R2IK_ABI_VERSION 6 /* 6: + symik_best_theta; 5: + symik_sweep; 4: + ctl_discrete_compact; 3: + symik_scalar, stream_synchronize, host pipelines, ctl_ctor_theta, reach_map_range_u16; no_limits / projected in elbow_positions, prev_joints in
+#define R2IK_ABI_VERSION 7 /* 7: + ctl_reach_map; 6: + symik_best_theta; 5: + symik_sweep; 4: + ctl_discrete_compact; 3: + symik_scalar, stream_synchronize, host pipelines, ctl_ctor_theta, reach_map_range_u16; no_limits / projected in elbow_positions, prev_joints in
                               no_limits, nullable `reachable`, test hook of the phased continuous entry as a parameter */
 
 /* argument errors */
@@ -368,6 +371,26 @@ int r2ik_reach_map_range_u16(r2ik_handle h, const double *origin, const double *
                              const double *orientations_euler /* device, n_ori x 3 */, int32_t ori_begin,
                              int32_t ori_end, int64_t voxel_begin, int64_t voxel_end, int32_t row_mod,
                              int32_t row_rem, uint16_t *counts, void *stream);
+
+/* The controller's workspace map: for each voxel v and the orientations o in [ori_begin, ori_end), the pose
+ * M(v, o) = [R_o | p_v; 0 0 0 1] with R_o = orientations[o] (row-major 3x3) and p_v = origin + (ix,iy,iz)*step, each
+ * coordinate a plain multiply then a plain add (no fused multiply-add), v = (ix*dims[1] + iy)*dims[2] + iz.
+ *   accepted[v]  = #o for which ControlIK.symbolic_inverse_kinematics(name, M(v, o), "discrete") returns
+ *                  reachable = True, i.e. r2ik_ctl_discrete_f64's `reachable` flag for that pose;
+ *   reachable[v] = #o for which is_reachable holds on the rotation the controller solves with (after the identity snap
+ *                  of control_ik.py:212-217), i.e. r2ik_ctl_discrete_f64's state in {REACHABLE, LIMITED_BY_SHOULDER}.
+ *                  Nullable.  accepted <= reachable; the difference is the "limited by shoulder" count.
+ * A block R_o with det <= 0 (INVALID_ROTATION) counts in neither.  The counts depend on the handle (arm, solver
+ * parameters, singularity_offset) and on par->preferred_theta (already mirrored for l_arm) and par->nb_search_points
+ * (>= 2) only: interval_limit (constrained_mode), d_theta_max, the previous and current joints act after the verdict
+ * in discrete mode (they change the joints and the emergency bits), and the map describes a controller that is not
+ * latched by an emergency stop.  Continuous mode never rejects a reachable pose and has no map of its own.
+ * origin / step / dims: host.  Both volumes are overwritten, not accumulated; orientation slices of one set add up to the
+ * whole set's volume. */
+int r2ik_ctl_reach_map_u32(r2ik_handle h, const R2ikCtlParams *par /* host */, const double *origin, const double *step,
+                           const int32_t *dims, const double *orientations /* device, n_ori x 9 row-major 3x3 */,
+                           int32_t ori_begin, int32_t ori_end, uint32_t *accepted, uint32_t *reachable /* nullable */,
+                           void *stream);
 
 /* Forward kinematics: M[i] (row-major 4x4) = tip pose in the torso frame for joints[i] (7).
  * chain: host pointer.  device: CUDA ordinal to launch on. */

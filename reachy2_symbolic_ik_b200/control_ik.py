@@ -163,6 +163,14 @@ class ControlIK:
         p.nb_search_points_continuous = 10
         return p
 
+    def reach_map(self, name: str, n: int = 256, orientations=None, n_orientations: int = 512, **kw):
+        """The controller's workspace map for arm ``name``: int32 CUDA tensor (n,n,n) of per-voxel counts of the
+        orientations that discrete mode accepts (``(accepted, reachable)`` with ``with_reachable=True``; see
+        ``workspace.ctl_reach_map``; all-reduced over ranks when ``dist=torch.distributed``)."""
+        from . import workspace
+
+        return workspace.ctl_reach_map(self, name, n=n, orientations=orientations, n_orientations=n_orientations, **kw)
+
     def _dev(self, x, shape=None):
         torch = self._torch
         t = torch.as_tensor(np.ascontiguousarray(x, dtype=np.float64) if not hasattr(x, "is_cuda") else x,

@@ -350,6 +350,60 @@ R2IK_HD bool disc_search(const SearchPlan &P, int nb, double &theta) {
 }
 
 // ---------------------------------------------------------------------------------------
+// The controller's workspace map (k_ctl_reach_map, r2ik_ctl_reach_map_u32): for a voxel centre p and an orientation R,
+// what discrete mode decides for the pose [R | p] -- the reference's `reachable` output and whether is_reachable held
+// on the rotation the controller solves with.  Neither depends on the joints the controller would go to, so the pair
+// stops after the elbow search: no discrete_finish, no safety chain.
+// ---------------------------------------------------------------------------------------
+// Grid coordinate o + i * s as a multiply then an add (no contraction into an FMA): the host can rebuild the voxel
+// centre, and so the pose, bit for bit.
+R2IK_HD double grid_coord(double o, int i, double s) {
+#if defined(__CUDA_ARCH__)
+  return __dadd_rn(o, __dmul_rn((double)i, s));
+#else
+  return o + (double)i * s;   // host builds compile with -ffp-contract=off
+#endif
+}
+
+// Per orientation: the rotation the controller solves with for the 3x3 block Rin (row-major) of a pose, i.e.
+// rotation_from_mat4 with the identity snap (ctl:212-217) on [Rin | 0]; it reads the 3x3 block only, so the result holds
+// for every voxel.  false: det <= 0 (INVALID_ROTATION; the pair is neither reachable nor accepted), R zeroed.
+R2IK_HD bool ctl_map_rotation(const double Rin[9], double R[9]) {
+  const double M[16] = {Rin[0], Rin[1], Rin[2], 0.0, Rin[3], Rin[4], Rin[5], 0.0, Rin[6], Rin[7], Rin[8], 0.0,
+                        0.0, 0.0, 0.0, 1.0};
+  if (rotation_from_mat4(M, true, R)) return true;
+  for (int k = 0; k < 9; ++k) R[k] = 0.0;
+  return false;
+}
+
+struct CtlPair {
+  bool reachable;   // is_reachable held: discrete mode's state is REACHABLE or LIMITED_BY_SHOULDER
+  bool accepted;    // discrete mode's `reachable` output: the preferred theta or a sample of the search passed is_elbow_ok
+};
+
+// Per (voxel, orientation) pair, R from ctl_map_rotation: the calls of disc_classify after the pose load (is_reachable,
+// then the preferred theta), then the search of k_ctl_discrete (disc_search on disc_search_plan), in the same order.
+// The first two are written out here rather than factored out of disc_classify: every way of sharing them that was
+// tried (the tail as a function taking Reach by reference or returning it) changed the code the compiler made for
+// k_disc_classify or k_ctl_discrete_scan (a larger stack frame, other register allocation).
+R2IK_HD CtlPair ctl_reach_pair(const ArmConst &A, const R2ikCtlParams &par, const double pos[3], const double R[9]) {
+  Solve S;
+  for (int k = 0; k < 9; ++k) S.R[k] = R[k];
+  const Reach rc = is_reachable_R<false>(A, pos, S);
+  CtlPair out;
+  out.reachable = rc.state == R2IK_STATE_REACHABLE;
+  out.accepted = false;
+  if (out.reachable) {
+    out.accepted = preferred_theta_works(A, S, rc.i0, rc.i1, par.preferred_theta);
+    if (!out.accepted) {
+      double theta;
+      out.accepted = disc_search(disc_search_plan(A, par, S, rc), par.nb_search_points, theta);
+    }
+  }
+  return out;
+}
+
+// ---------------------------------------------------------------------------------------
 // Continuous mode (ctl:276-407), cut at its data dependences.  Of one waypoint's work only two thin
 // strands depend on the trajectory's past: the rate-limited elbow angle (previous_theta) and the
 // unwrap / continuity / emergency chain (previous_sol).  Everything else -- the goal rotation,

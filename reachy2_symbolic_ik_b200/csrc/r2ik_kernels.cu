@@ -12,6 +12,7 @@
 //                                               and per-trajectory scans;  k_ctl_continuous = the one-kernel form
 //   K4     k_reach_map                          one thread / voxel, mixed-precision flag with FP64 escalation
 //          k_reach_map_f64                      every pair by the FP64 flag solve (cross-check)
+//   K4c    k_ctl_reach_map                      one thread / voxel, ControlIK discrete mode's verdict per orientation
 //
 // The work is scalar FP64 / FP32 (sincos / atan2 / sqrt / FMA chains): it runs on the FP64 and FP32 pipes, not on
 // tensor cores; HBM traffic is a few hundred bytes per pose.  There is no host implementation
@@ -745,6 +746,85 @@ k_reach_map_f64(const __grid_constant__ ArmConst A, double ox, double oy, double
 }
 
 // ---------------------------------------------------------------------------------------
+// K4c: the controller's workspace map.  accepted[v] = number of orientations for which ControlIK's discrete mode returns
+// reachable = True for the pose [R_o | voxel centre], reachable[v] (nullable) = number for which is_reachable holds on
+// the rotation the controller solves with.  K4's shape: one thread per voxel, a block without a voxel that passes the
+// pre-checks (they depend on the position alone and are the first step of is_reachable, so such a voxel counts 0 for
+// every orientation) leaves before staging anything, and the rotations (identity snap / literal route of
+// rotation_from_mat4, ctl_map_rotation) are staged per chunk of R2IK_ORI_CHUNK orientations in shared memory.  Each pair
+// runs ctl_reach_pair (r2ik_control.cuh): is_reachable, the preferred theta, the K-sample search.
+// ---------------------------------------------------------------------------------------
+// Held to 128 registers (4 blocks / SM, 8 B of spills): 108.9 ms per 256^3 x 512 (r_arm, K = 20) against 134.6 ms at the
+// 144 registers the compiler picks unconstrained (3 blocks) and 117.9 ms at 64 registers (~430 B of spills; the 37 KB
+// of staged rotations allow 6 blocks / SM), NVIDIA B200 at 1000 W, profiles/r5_exp_ctl_reach_map_mb{1,4,8}.txt.
+#ifndef R2IK_K4C_MINBLOCKS
+#define R2IK_K4C_MINBLOCKS 4
+#endif
+__global__ void __launch_bounds__(R2IK_BLOCK, R2IK_K4C_MINBLOCKS)
+k_ctl_reach_map(const __grid_constant__ ArmConst A, const __grid_constant__ R2ikCtlParams par, double ox, double oy,
+                double oz, double sx, double sy, double sz, int d1, int d2, int64_t nv, const double *__restrict__ ori,
+                int ori_begin, int ori_end, uint32_t *__restrict__ accepted, uint32_t *__restrict__ reachable) {
+  __shared__ double sR[R2IK_ORI_CHUNK][9];
+  __shared__ uint8_t sOk[R2IK_ORI_CHUNK];
+  const int64_t v = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  double pos[3] = {0.0, 0.0, 0.0};
+  bool live = false;
+  if (v < nv) {
+    int ix, iy, iz;
+    if (nv <= 0x7fffffffLL) {
+      const unsigned u = (unsigned)v, row = u / (unsigned)d2;
+      iz = (int)(u - row * (unsigned)d2);
+      ix = (int)(row / (unsigned)d1);
+      iy = (int)(row - (unsigned)ix * (unsigned)d1);
+    } else {
+      iz = (int)(v % d2);
+      iy = (int)((v / d2) % d1);
+      ix = (int)(v / ((int64_t)d2 * d1));
+    }
+    pos[0] = grid_coord(ox, ix, sx); pos[1] = grid_coord(oy, iy, sy); pos[2] = grid_coord(oz, iz, sz);
+    double px = pos[0], py = pos[1], pz = pos[2];
+    live = reach_prechecks(A, px, py, pz) < 0;
+  }
+  if (!__syncthreads_or(live ? 1 : 0)) {
+    if (v < nv) {
+      accepted[v] = 0;
+      if (reachable) reachable[v] = 0;
+    }
+    return;
+  }
+  uint32_t n_acc = 0, n_reach = 0;
+  for (int base = ori_begin; base < ori_end; base += R2IK_ORI_CHUNK) {
+    const int m = min(R2IK_ORI_CHUNK, ori_end - base);
+    if (base != ori_begin) __syncthreads();
+    for (int o = threadIdx.x; o < m; o += blockDim.x) {
+      const double *r = ori + 9 * (size_t)(base + o);
+      double Rin[9], R[9];
+#pragma unroll
+      for (int k = 0; k < 9; ++k) Rin[k] = r[k];
+      sOk[o] = ctl_map_rotation(Rin, R) ? 1 : 0;
+#pragma unroll
+      for (int k = 0; k < 9; ++k) sR[o][k] = R[k];
+    }
+    __syncthreads();
+    if (live) {
+      for (int o = 0; o < m; ++o) {
+        if (!sOk[o]) continue;
+        double R[9];
+#pragma unroll
+        for (int k = 0; k < 9; ++k) R[k] = sR[o][k];
+        const CtlPair c = ctl_reach_pair(A, par, pos, R);
+        n_reach += c.reachable ? 1u : 0u;
+        n_acc += c.accepted ? 1u : 0u;
+      }
+    }
+  }
+  if (v < nv) {
+    accepted[v] = n_acc;
+    if (reachable) reachable[v] = n_reach;
+  }
+}
+
+// ---------------------------------------------------------------------------------------
 __device__ __forceinline__ void affine_mul(double A[12], const double B[12]) {
   double o[12];
 #pragma unroll
@@ -1315,6 +1395,29 @@ int r2ik_reach_map_f64_u32(r2ik_handle h, const double *origin, const double *st
                            const double *orientations_euler, int32_t ori_begin, int32_t ori_end, uint32_t *counts,
                            void *stream) {
   return reach_map_launch(true, h, origin, step, dims, orientations_euler, ori_begin, ori_end, counts, stream);
+}
+
+int r2ik_ctl_reach_map_u32(r2ik_handle h, const R2ikCtlParams *par, const double *origin, const double *step,
+                           const int32_t *dims, const double *orientations, int32_t ori_begin, int32_t ori_end,
+                           uint32_t *accepted, uint32_t *reachable, void *stream) {
+  if (!h || !par) return fail_arg(R2IK_ERR_NULL, "r2ik_ctl_reach_map_u32: null handle or parameters");
+  if (par->nb_search_points < 2) return fail_arg(R2IK_ERR_ARG, "r2ik_ctl_reach_map_u32: bad nb_search_points");
+  if (!origin || !step || !dims || !orientations || !accepted)
+    return fail_arg(R2IK_ERR_NULL, "r2ik_ctl_reach_map_u32: null argument");
+  if (dims[0] <= 0 || dims[1] <= 0 || dims[2] <= 0 || ori_begin < 0 || ori_end < ori_begin)
+    return fail_arg(R2IK_ERR_ARG, "r2ik_ctl_reach_map_u32: bad dims or orientation range");
+  const int64_t plane = (int64_t)dims[1] * dims[2], max_voxels = (int64_t)0x7fffffff * R2IK_BLOCK;
+  if (plane > max_voxels / dims[0])
+    return fail_arg(R2IK_ERR_ARG, "r2ik_ctl_reach_map_u32: volume larger than one launch can cover");
+  const int64_t nv = dims[0] * plane;
+  DeviceGuard guard_(h->device);
+  R2IK_CUDA(guard_.err, "cudaSetDevice");
+  k_ctl_reach_map<<<blocks_for(nv), R2IK_BLOCK, 0, (cudaStream_t)stream>>>(h->A, *par, origin[0], origin[1], origin[2],
+                                                                          step[0], step[1], step[2], dims[1], dims[2], nv,
+                                                                          orientations, ori_begin, ori_end, accepted,
+                                                                          reachable);
+  R2IK_CUDA(cudaGetLastError(), "k_ctl_reach_map launch");
+  return 0;
 }
 
 int r2ik_fk_f64(const R2ikFkChain *chain, int device, const double *joints, int64_t n, double *M, void *stream) {

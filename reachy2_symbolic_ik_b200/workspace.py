@@ -5,6 +5,10 @@ The reference has no such component; its closest code is the task-space grid swe
 voxel grid x orientation set is swept by the K4 kernel (``r2ik_reach_map_u32``): counts[v] =
 number of orientations for which ``SymbolicIK.is_reachable(voxel centre, orientation)`` is True.
 
+``ctl_reach_map`` is the same sweep for ``ControlIK``'s discrete mode (``r2ik_ctl_reach_map_u32``): counts[v] = number
+of orientations for which the controller accepts the pose, i.e. is_reachable holds AND an elbow angle passes
+``is_elbow_ok`` (the preferred one or a sample of the search).
+
 Multi-GPU: poses / trajectories are independent, so batches are cut into contiguous slices
 (``shard_range``) with no exchange.  The reach map shards the ORIENTATION set; every rank counts its
 shard for every voxel and the volumes are summed by an all-reduce (NCCL over NVLink / NVSwitch) -- the
@@ -194,6 +198,91 @@ def reach_map(solver, n: int = 256, orientations_euler=None, n_orientations: int
             return out
 
         return sharded_sum(launch, n_ori, dist, group, mark)
+
+
+def rpy_matrices(euler) -> np.ndarray:
+    """(n, 3) xyz Euler angles (roll, pitch, yaw) -> (n, 3, 3) rotation matrices Rz(yaw) Ry(pitch) Rx(roll): the
+    vectorised ``fk._rpy_matrix``."""
+    e = np.asarray(euler, dtype=np.float64).reshape(-1, 3)
+    cr, sr = np.cos(e[:, 0]), np.sin(e[:, 0])
+    cp, sp = np.cos(e[:, 1]), np.sin(e[:, 1])
+    cy, sy = np.cos(e[:, 2]), np.sin(e[:, 2])
+    R = np.empty((len(e), 3, 3))
+    R[:, 0, 0] = cy * cp; R[:, 0, 1] = cy * sp * sr - sy * cr; R[:, 0, 2] = cy * sp * cr + sy * sr
+    R[:, 1, 0] = sy * cp; R[:, 1, 1] = sy * sp * sr + cy * cr; R[:, 1, 2] = sy * sp * cr - cy * sr
+    R[:, 2, 0] = -sp; R[:, 2, 1] = cp * sr; R[:, 2, 2] = cp * cr
+    return R
+
+
+def orientation_matrices(orientations) -> np.ndarray:
+    """An orientation set as (n, 3, 3) float64 rotation matrices: (n, 3, 3) matrices are taken as given, (n, 3) xyz
+    Euler angles go through ``rpy_matrices``."""
+    o = orientations.detach().cpu().numpy() if hasattr(orientations, "detach") else np.asarray(orientations)
+    o = np.asarray(o, dtype=np.float64)
+    if o.ndim == 3 and o.shape[1:] == (3, 3):
+        return np.ascontiguousarray(o)
+    if o.ndim == 2 and o.shape[1] == 3:
+        return rpy_matrices(o)
+    raise ValueError(f"orientations must be (n, 3, 3) rotation matrices or (n, 3) xyz Euler angles, got {o.shape}")
+
+
+def ctl_reach_map(controller, name: str, n: int = 256, orientations=None, n_orientations: int = 512,
+                  preferred_theta: float = -4 * np.pi / 6, origin=None, step=None, dims=None, with_reachable: bool = False,
+                  dist=None, group=None, out=None, mark=None):
+    """The controller's workspace map (``r2ik_ctl_reach_map_u32``): for ``controller`` (a ``ControlIK``) and arm ``name``,
+    the int32 CUDA volume (d0, d1, d2) of per-voxel counts of the orientations for which
+    ``controller.symbolic_inverse_kinematics_batch(name, M, "discrete", preferred_theta=preferred_theta)`` returns
+    reachable = True, M = [R_o | voxel centre].  Voxel centres are origin + (ix, iy, iz) * step (a multiply then an add,
+    no fused multiply-add); the default grid is ``reach_grid`` with n cells per side.
+
+    orientations: (n_ori, 3, 3) rotation matrices, or (n_ori, 3) xyz Euler angles (``rpy_matrices``); default
+    ``fibonacci_orientations(n_orientations)``.  A block with det <= 0 counts nowhere.
+    with_reachable: return (accepted, reachable), where reachable counts the orientations for which ``is_reachable``
+    holds on the rotation the controller solves with (discrete state REACHABLE or LIMITED_BY_SHOULDER); reachable -
+    accepted is the per-voxel "limited by shoulder" count.  Both come out of the same pass.
+    The counts depend on the arm, the controller's solver (``is_dvt``), ``controller.nb_search_points`` and
+    ``preferred_theta`` (mirrored for l_arm as in the batched call).  They do not depend on ``constrained_mode``,
+    ``d_theta_max``, ``previous_joints`` or ``current_joints``, which in discrete mode only change the joints and the
+    emergency bits, so they are not parameters here; the map describes a controller that is not latched by
+    ``emergency_stop``.  Continuous mode never rejects a reachable pose and has no map of its own.
+    dist: an initialised ``torch.distributed``; each rank counts its slice of the orientation set and one int32
+    all-reduce sums the volumes (both at once when ``with_reachable``); every rank returns the full map.
+    out: int32 CUDA tensor (2, d0, d1, d2) with ``with_reachable``, else (d0, d1, d2), reused for the result."""
+    torch = controller._torch
+    solver = controller.symbolic_ik_solver[name]
+    par = controller._ctl_params(name, "unconstrained", preferred_theta, 0.01)
+    if orientations is None:
+        orientations = fibonacci_orientations(n_orientations)
+    if origin is None or step is None or dims is None:
+        origin, step, dims = reach_grid(solver.shoulder_position, solver.max_arm_length, n)
+    origin = np.ascontiguousarray(origin, dtype=np.float64)
+    step = np.ascontiguousarray(step, dtype=np.float64)
+    dims = np.ascontiguousarray(dims, dtype=np.int32)
+    shape = tuple(int(d) for d in dims)
+    dev = solver._device
+    with torch.cuda.device(dev):
+        ori = torch.from_numpy(orientation_matrices(orientations).reshape(-1, 9)).to(dev)
+        n_ori = ori.shape[0]
+        want = (2,) + shape if with_reachable else shape
+        if out is None:
+            out = torch.empty(want, dtype=torch.int32, device=dev)
+        elif tuple(out.shape) != want or out.dtype != torch.int32 or not out.is_contiguous() or out.device != dev:
+            raise ValueError(f"out must be a contiguous int32 tensor of shape {want} on {dev}")
+        acc = out[0] if with_reachable else out
+        reach = out[1] if with_reachable else None
+        dp = C.POINTER(C.c_double)
+
+        def launch(b: int, e: int):
+            s = torch.cuda.current_stream(dev).cuda_stream
+            rc = solver._handle.lib.r2ik_ctl_reach_map_u32(
+                solver._handle.h, C.byref(par), origin.ctypes.data_as(dp), step.ctypes.data_as(dp),
+                dims.ctypes.data_as(C.POINTER(C.c_int32)), C.c_void_p(ori.data_ptr()), C.c_int32(b), C.c_int32(e),
+                C.c_void_p(acc.data_ptr()), C.c_void_p(reach.data_ptr() if reach is not None else None), C.c_void_p(s))
+            _native.check(rc, "r2ik_ctl_reach_map_u32")
+            return out
+
+        sharded_sum(launch, n_ori, dist, group, mark)
+    return (acc, reach) if with_reachable else acc
 
 
 def task_space_grid(shoulder_position, arm_length: float = 0.5, x_step: float = 0.15, y_step: float = 0.15,
