@@ -645,6 +645,11 @@ R2IK_HD Reach solve_core_impl(const ArmConst &A, Solve &S) {
     const double rr = r2 * rho2;
     const double dl = rr - Xc * Xc;                       // sign of the reference's discriminant
     bool deg = fabs(n1[1]) < 1e-7 && fabs(n1[2]) < 1e-7;  // utl:66-70 special cases of rmfv(nL)
+    // ... and of rmfv(n2): within its isclose band a1, a2 are e_y, +-e_z, up to 1e-8 rad off the plane normal to n2, so
+    // X(theta) leaves the forearm sphere and the angles where it crosses the limit plane are not the reference's, which
+    // converts the true intersection points with that frame.  (The flag pass needs no frame: rho2 = 1 - Ca^2 is exact.)
+    // Tested on the high words, off the FP64 pipe: both |n2[1]|, |n2[2]| < 2^-24 (6e-8), a superset of the band.
+    if (!FLAG_ONLY) deg = deg || ((hi_word(n2[1]) & 0x7fffffff) < 0x3e700000 && (hi_word(n2[2]) & 0x7fffffff) < 0x3e700000);
     deg = deg || !(rho2 > 1e-12);                         // sik:475-483 (|n2 -+ n1| < 1e-7 componentwise => rho2 < 3e-14)
     deg = deg || fabs(Xc - nb) <= 1e-8 + 1e-5 * fabs(nb); // superset of np.isclose(u, t), sik:581: u - t = (Xc - nb) / rho
     deg = deg || !(r2 > 0.0) || fabs(dl) <= 1e-12 * (rr + Xc * Xc);
